@@ -2,6 +2,7 @@
 """bench.py - throughput of the decode -> sample -> preprocess -> embed/classify hot path on B200.
 
     python bench.py --gpus 1 --steps K --warmup W                 # this repo's CUDA path
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR  # ... and what its last timed step returned, as DIR/*.npy
     python bench.py --impl reference --gpus 1 --steps K --warmup W # the reference's CPU path (oracle) on host cores
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
@@ -10,6 +11,11 @@ residual-coded Intra16x16 IDRs + P pictures, CAVLC, deblocking on - no encoder e
 rank, sampled at 1 fps like AestheticFilterStage (11 frames per clip), CLIP ViT-L/14 image tower (seeded random weights) +
 aesthetic affine head.  One STEP = `--clips-per-step` clips (default 24 -> 264 frames, the closest whole-clip count to the
 256-frame batch BASELINE.json names).
+
+--dump-outputs writes what the last timed step returned (rank 0) in float32, one row per sampled frame in slot order (clip j's
+frames_per_clip frames at rows j * frames_per_clip ...): embedding.npy [frames_per_step, 768] and aesthetic_score.npy
+[frames_per_step].  The inputs are seeded (clips, weights), so two builds run with the same arguments can be compared output for
+output.
 
 Printed JSON line (rank 0):
   value   clips/s, whole job, decoded NV12 surfaces of the step already resident in HBM (preprocess + tower + head),
@@ -33,6 +39,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 from pathlib import Path
@@ -46,6 +53,7 @@ import numpy as np  # noqa: E402
 FRAME_W, FRAME_H, FPS, SECONDS = 1920, 1080, 30, 10.0
 SAMPLE_FPS = 1.0
 FALLBACK_PEAKS = {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0}
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 def peaks() -> tuple[dict, str]:
@@ -112,10 +120,10 @@ def _gen_clip(args) -> str:
 
 def make_clips(n_distinct: int, rank: int, workers: int | None = None, size: tuple[int, int] = (FRAME_W, FRAME_H), bitrate: float = BITRATE) -> list[bytes]:
     """`n_distinct` residual-coded clips (seed = 1000 * rank + i), generated by a fork pool BEFORE CUDA is initialised and
-    cached under /tmp (both arms of one box reuse them)."""
+    cached in the temporary directory (both arms on one machine reuse them)."""
     import multiprocessing as mp
 
-    root = os.path.join(os.environ.get("CB_CLIP_CACHE", "/tmp"), f"cb_clips_{size[0]}x{size[1]}_{FPS}_{int(SECONDS)}s_{int(bitrate)}")
+    root = os.path.join(os.environ.get("CB_CLIP_CACHE", tempfile.gettempdir()), f"cb_clips_{size[0]}x{size[1]}_{FPS}_{int(SECONDS)}s_{int(bitrate)}")
     os.makedirs(root, exist_ok=True)
     jobs = [(1000 * rank + i, os.path.join(root, f"clip_{1000 * rank + i}.mp4"), size[0], size[1], bitrate) for i in range(n_distinct)]
     todo = [j for j in jobs if not os.path.exists(j[1])]
@@ -247,6 +255,8 @@ def run_b200(args) -> None:
 
     stage = make_stage(seek=False)
     ctx = get_context()
+    backend = ctx.decode_backend()  # "libavcodec" (host) where the driver exposes no NVDEC engine: every decode figure below is then host decode
+    decoder = "NVDEC" if backend == "nvdec" else "libavcodec host decode (no NVDEC engine exposed)"
     tower = model.tower
 
     def make_tasks(call: int) -> list:
@@ -301,6 +311,8 @@ def run_b200(args) -> None:
     barrier()
     dev_s = max_over_ranks(ev0.elapsed_time(ev1) / 1e3)
     launches = ctx.launch_count() - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"embedding": emb, "aesthetic_score": score})
     value = world * cps * args.steps / dev_s
     del pool0
 
@@ -332,7 +344,7 @@ def run_b200(args) -> None:
                 "api": "NvdecClipAestheticStage.process_data(list[SplitPipeTask]) on a set-up stage (the call xenna's StageWorker makes)",
                 "clips_per_call": cps * args.tasks_per_call, "calls": n_calls, "ms_per_call": 1e3 * sec / n_calls,
                 "frames_per_sec": world * n_clips * fpc / sec, "decoded_frames_per_sec": decoded_all / sec,
-                "decoded_frames_per_clip": decoded / max(1, n_clips), "nvdec_sessions": args.decoders,
+                "decoded_frames_per_clip": decoded / max(1, n_clips), "decode_backend": backend, "decode_sessions": args.decoders,
                 "stage_perf_process_time_s": perf_s, "wall_s_this_rank": wall_local,
                 "host_cpu_cores_busy_this_rank": cpu_used / wall_local, "numa_node": st.last_call_stats.get("numa_node"),
                 "pinned_cpus": st.last_call_stats.get("pinned_cpus"), "seek_keyframes": bool(st._seek)}  # fmt: skip
@@ -378,7 +390,7 @@ def run_b200(args) -> None:
                 fps_real = decode_only(stage._decode_pool, [sd], 3.0)
                 real = {"clip": "tests/golden/sintel_clip_10s.mp4 (854x480, High profile, CABAC, B-frames-free real content)", "frames_per_sec_per_gpu": fps_real,
                         "macroblocks_per_sec": fps_real * 54 * 30, "as_1080p_frames_per_sec": fps_real * (54 * 30) / (120 * 68)}  # fmt: skip
-            ceiling = {"decode_only_frames_per_sec_per_gpu": ceil_fps, "seconds": args.ceiling_seconds, "sessions": args.decoders,
+            ceiling = {"decoder": decoder, "decode_only_frames_per_sec_per_gpu": ceil_fps, "seconds": args.ceiling_seconds, "sessions": args.decoders,
                        "e2e_fraction_of_decode_ceiling": (e2e["decoded_frames_per_sec"] / world) / ceil_fps if ceil_fps > 0 else None,
                        "real_content": real}  # fmt: skip
             stage.destroy()
@@ -446,13 +458,13 @@ def run_b200(args) -> None:
         "metric": "clips_per_sec", "value": value, "unit": "clips/s", "n_gpus": world, "steps": args.steps, "warmup": max(args.warmup, 3), "ms_per_step": step_ms,
         "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f16", "data": "synthetic",
         "frames_per_sec": world * frames_per_step * args.steps / dev_s,
-        "config": {"workload": WORKLOAD, "implementation": "one process per B200: NVDEC + fused preprocess kernel + tcgen05 tower behind NvdecClipAestheticStage",
+        "config": {"workload": WORKLOAD, "implementation": f"one process per B200: {decoder} + fused preprocess kernel + tcgen05 tower behind NvdecClipAestheticStage",
                    "clips_per_step": cps, "frames_per_clip": fpc, "frames_per_step": frames_per_step, "sample_fps": SAMPLE_FPS, "distinct_clips": args.distinct_clips,
                    "clip_bitrate_bps": float(np.mean([8 * len(c) / SECONDS for c in clips])),
                    "clip_stream": "tools/synth_h264.make_coded_clip: Intra16x16 IDR (DC + sparse AC, chroma DC) + P (P_Skip runs, quarter-pel 16x16 motion, sparse 4x4 residuals), CAVLC, deblocking on, GOP 30",
                    "network": "clip-vit-large-patch14, seeded random weights, fp16 operands / fp32 accumulate+residual", "sharding": f"{world} rank(s), clips sharded per rank, no data-path collective",
                    "l2": "inputs (NV12 pool 0.88 GB + activations > 1 GB) exceed the 126 MB L2", "value_inputs": "decoded NV12 surfaces resident in HBM"},
-        "clocks": clocks, "gpu_launches": int(launches),
+        "decode_backend": backend, "clocks": clocks, "gpu_launches": int(launches),
         "roofline": {"bound": "tensor", "kernel": "gemm_tcgen05_2cta_kernel", "achieved": ach_tf, "peak": peak_tf, "unit": "TFLOP/s", "frac": ach_tf / peak_tf,
                      "traffic": traffic.get("gemm_tcgen05_2cta"), "traffic_source": traffic.get("_source"),
                      "peak_source": f"{pk_src} bf16_tflops_sustained (kernel timed inside a long step)", "launches_per_step": gemm_n / args.steps,
@@ -472,7 +484,7 @@ def run_b200(args) -> None:
         line["e2e_error"] = e2e_error
     if world == 1 and not args.no_secondary:
         try:
-            line["secondary"] = secondary_configs(ctx, torch, clips, clips_4k, args, clips_720)
+            line["secondary"] = secondary_configs(ctx, torch, clips, clips_4k, args, clips_720, decoder)
         except Exception as exc:  # noqa: BLE001
             import traceback
 
@@ -489,7 +501,22 @@ def run_b200(args) -> None:
         dist.destroy_process_group()
 
 
-def secondary_configs(ctx, torch, clips_1080p: list[bytes], clips_4k, args, clips_720=None) -> dict:
+def dump_outputs(out_dir: str, outputs: dict) -> None:
+    """Write each output as out_dir/<name>.npy in float32.  The outputs share their leading (frame) dimension; above
+    DUMP_LIMIT_BYTES in all, the same seeded sample of rows is kept from each and its row indices go to sample_rows.npy."""
+    arrays = {name: t.detach().float().cpu().numpy() for name, t in outputs.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        n = next(iter(arrays.values())).shape[0]
+        rows = np.sort(np.random.default_rng(0).choice(n, size=DUMP_LIMIT_BYTES // (total // n + 8), replace=False))
+        arrays = {name: a[rows] for name, a in arrays.items()}
+        arrays["sample_rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
+def secondary_configs(ctx, torch, clips_1080p: list[bytes], clips_4k, args, clips_720=None, decoder: str = "NVDEC") -> dict:
     """Bounded secondary rows (N=1, rank 0): BASELINE.json configs[0] (C1) on both arms, a configs[3]-shaped row (4K + SoViT-400m) and
     the transcode-free clip cutter.  Not the headline; each states its own workload."""
     import uuid
@@ -599,7 +626,7 @@ def secondary_configs(ctx, torch, clips_1080p: list[bytes], clips_4k, args, clip
                         "filter (BASELINE.json configs[4] mix on one GPU; the reference's split / caption / writer stages around it are out of scope)",
             "e2e_clips_per_sec": cps, "clips": n, "decoded_megapixels_per_sec": cps * 300 * mean_px / 1e6,
             "kernel_ms_over_warmup_and_timed_call": {k: v["ms"] for k, v in prof.items() if v["launches"] and k != "other"},  # "other" would absorb the idle gaps while the SMs wait for NVDEC
-            "note": "compare decoded_megapixels_per_sec with the 1080p ceiling (decode_roofline.decode_only_frames_per_sec x 2.07 Mpx); one NVDEC session per stream shape per "
+            "note": f"decoder: {decoder}; compare decoded_megapixels_per_sec with the 1080p ceiling (decode_roofline.decode_only_frames_per_sec x 2.07 Mpx); one decode session per stream shape per "
                     "worker thread - a session that is fed another resolution is destroyed and re-created by the driver (tools/mixed_decode_probe.py)"}  # fmt: skip
 
     # ---- video-tower input tubes (N5, formulation only): 1080p clips -> 2 fps -> 8 kept frames -> cv2-bilinear 224 x 224 + ImageNet normalise
@@ -627,7 +654,7 @@ def secondary_configs(ctx, torch, clips_1080p: list[bytes], clips_4k, args, clip
                     "(InternVideo2FrameCreationStage, source=nvdec; the tower itself is not part of this path)",
         "e2e_clips_per_sec": cps, "clips": n, "d2h_bytes_per_clip": 8 * 3 * 224 * 224 * 4,
         "kernel": {"ms_per_256_frames": ms, "algorithmic_gbs": tube_b / (ms / 1e3) / 1e9, "bound": "hbm (sparse: 4 source pixels per output; sector-granular reads)"},
-        "note": "NVDEC-bound like the headline: every frame up to the last kept one is decoded"}  # fmt: skip
+        "note": f"decode-bound ({decoder}) like the headline: every frame up to the last kept one is decoded"}  # fmt: skip
 
     # ---- transcode-free clip cutting (N2): 5 s spans out of the 10 s 1080p sources by stream copy
     stage = ClipStreamCopyStage()
@@ -825,7 +852,12 @@ def main() -> None:
     ap.add_argument("--no-shots", action="store_true", help="skip the shot-detection secondary measurement")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's per-frame embeddings and aesthetic scores (rank 0) as DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -23,6 +23,7 @@ ACT_QUICK_GELU, ACT_GELU_TANH = 0, 1
 ARCH_CLIP, ARCH_SIGLIP = 0, 1
 EPI_NONE, EPI_QUICK_GELU, EPI_GELU_TANH = 0, 1, 2
 DECODE_SEEK_SYNC, DECODE_DISCARD_ALL = 1, 2
+DECODE_BACKENDS = {0: "nvdec", 1: "libavcodec"}
 CUBIC_OPENCV, CUBIC_IPP = 0, 1
 
 
@@ -91,6 +92,7 @@ SIGNATURES = {
     "cb_affine_score": (_i, [_vp, _vp, _vp, _f, _vp, _i, _i, _vp]),
     "cb_mp4_index": (_i, [_vp, _vp, C.c_size_t, C.POINTER(Mp4Info), C.POINTER(C.c_int64), C.POINTER(C.c_uint8), _i]),
     "cb_mp4_cut": (_i, [_vp, _vp, C.c_size_t, _i, _i, _vp, C.c_size_t, C.POINTER(C.c_size_t)]),
+    "cb_decode_backend": (_i, [_vp, C.POINTER(_i)]),
     "cb_decoder_create": (_i, [_vp, C.POINTER(_vp)]),
     "cb_decoder_destroy": (None, [_vp]),
     "cb_decoder_decode": (_i, [_vp, _vp, C.c_size_t, _pi32, _i, C.POINTER(SurfacePool), _pi32, C.POINTER(DecodeStats)]),

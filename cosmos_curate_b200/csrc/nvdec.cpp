@@ -22,6 +22,7 @@
 
 #include "common.h"
 #include "mp4_demux.h"
+#include "swdec.h"
 
 namespace {
 
@@ -104,6 +105,18 @@ struct CUVIDDECODECREATEINFO {
 };
 static_assert(sizeof(CUVIDDECODECREATEINFO) == 176, "CUVIDDECODECREATEINFO layout");
 
+struct CUVIDDECODECAPS {
+  int eCodecType, eChromaFormat;
+  unsigned nBitDepthMinus8, reserved1[3];
+  unsigned char bIsSupported, nNumNVDECs;
+  unsigned short nOutputFormatMask;
+  unsigned nMaxWidth, nMaxHeight, nMaxMBCount;
+  unsigned short nMinWidth, nMinHeight;
+  unsigned char bIsHistogramSupported, nCounterBitDepth;
+  unsigned short nMaxHistogramBins;
+  unsigned reserved3[10];
+};
+
 struct CUVIDPROCPARAMS {
   int progressive_frame, second_field, top_field_first, unpaired_field;
   unsigned reserved_flags, reserved_zero;
@@ -130,6 +143,7 @@ struct CuvidApi {
   int (*UnmapVideoFrame64)(CUvideodecoder, unsigned long long) = nullptr;
   int (*CtxLockCreate)(CUvideoctxlock*, void* /*CUcontext*/) = nullptr;
   int (*CtxLockDestroy)(CUvideoctxlock) = nullptr;
+  int (*GetDecoderCaps)(CUVIDDECODECAPS*) = nullptr;  // optional: only used to find out whether the device has an engine
   std::string error;
 };
 
@@ -160,12 +174,14 @@ CuvidApi* load_cuvid() {
     CB_SYM(CtxLockCreate, "cuvidCtxLockCreate")
     CB_SYM(CtxLockDestroy, "cuvidCtxLockDestroy")
 #undef CB_SYM
+    *(void**)(&api.GetDecoderCaps) = dlsym(api.handle, "cuvidGetDecoderCaps");
   });
   return &api;
 }
 
 struct NvdecShared {  // per cb_ctx
   CUvideoctxlock lock = nullptr;
+  bool software = false;  // the driver exposes no NVDEC engine to this process: sessions decode with libavcodec (swdec.h)
 };
 
 }  // namespace
@@ -194,6 +210,14 @@ struct cb_decoder {
   int thumb_w = 0, thumb_h = 0, thumb_cap = 0;
   std::string error;
   std::vector<uint8_t> scratch;
+  // host decode (NvdecShared::software): libavcodec session, NV12 staging on the host and in device memory
+  bool software = false;
+  cb::SwDecoder* sw = nullptr;
+  int sw_codec = -1;
+  bool sw_low_delay = false;
+  std::vector<uint8_t> sw_host;
+  uint8_t* sw_dev = nullptr;
+  size_t sw_dev_bytes = 0;
 };
 
 namespace {
@@ -259,6 +283,47 @@ int on_decode(void* user, void* pic) {
   return 1;
 }
 
+// One displayed picture, NV12 in device memory (luma rows rounded up to even, then the chroma rows) at `pitch`: scaled into
+// the thumbnail output, or copied into every surface slot that asked for display index `idx`.
+int deliver(cb_decoder* d, int idx, const uint8_t* src, size_t pitch) {
+  if (d->thumb_out) {
+    const int th = (d->disp_h + 1) & ~1;
+    int trc = cb::bilinear_from_surface(d->ctx, src, (int)pitch, th, d->disp_w, d->disp_h, d->thumb_w, d->thumb_h,
+                                        d->thumb_out + (size_t)idx * d->thumb_w * d->thumb_h * 3, d->stream);
+    cudaError_t te = cudaStreamSynchronize(d->stream);
+    if (trc != 0 || te != cudaSuccess) {
+      d->error = "thumbnail kernel failed";
+      return 0;
+    }
+    d->emitted++;
+    return 1;
+  }
+  if (((d->disp_w + 1) & ~1) != d->dst_w || ((d->disp_h + 1) & ~1) != d->dst_h) {
+    d->error = "clip is " + std::to_string(d->disp_w) + "x" + std::to_string(d->disp_h) + " but the surface pool is " + std::to_string(d->dst_w) +
+               "x" + std::to_string(d->dst_h);
+    return 0;
+  }
+  const int th = d->dst_h;  // target height (even)
+  cudaError_t e = cudaSuccess;
+  while (d->next_id < d->n_ids && d->ids[d->next_id] == idx) {  // a repeated id (supersampling) fills several slots
+    uint8_t* dst = d->dst_base + (size_t)d->slots[d->next_id] * d->dst_slot_stride;
+    e = cudaMemcpy2DAsync(dst, d->dst_pitch, src, pitch, d->dst_w, th, cudaMemcpyDeviceToDevice, d->stream);
+    if (e == cudaSuccess)
+      e = cudaMemcpy2DAsync(dst + (size_t)d->dst_luma_rows * d->dst_pitch, d->dst_pitch, src + pitch * th, pitch, d->dst_w, th / 2,
+                            cudaMemcpyDeviceToDevice, d->stream);
+    if (e != cudaSuccess) break;
+    d->next_id++;
+    d->emitted++;
+  }
+  if (e == cudaSuccess) e = cudaStreamSynchronize(d->stream);  // the source must outlive the copy
+  if (e != cudaSuccess) {
+    d->error = std::string("surface copy failed: ") + cudaGetErrorString(e);
+    return 0;
+  }
+  if (d->next_id >= d->n_ids) d->done = true;
+  return 1;
+}
+
 int on_display(void* user, CUVIDPARSERDISPINFO* info) {
   cb_decoder* d = (cb_decoder*)user;
   if (!info || d->done) return 1;
@@ -275,33 +340,8 @@ int on_display(void* user, CUVIDPARSERDISPINFO* info) {
       d->done = true;
       return 1;
     }
-    CUVIDPROCPARAMS tp;
-    memset(&tp, 0, sizeof tp);
-    tp.progressive_frame = info->progressive_frame, tp.top_field_first = info->top_field_first, tp.output_stream = d->stream;
-    unsigned long long tsrc = 0;
-    unsigned tpitch = 0;
-    int trc = d->api->MapVideoFrame64(d->dec, info->picture_index, &tsrc, &tpitch, &tp);
-    if (trc != 0) {
-      d->error = "cuvidMapVideoFrame64 failed with CUresult " + std::to_string(trc);
-      return 0;
-    }
-    const int th = (d->disp_h + 1) & ~1;
-    trc = cb::bilinear_from_surface(d->ctx, (const void*)tsrc, (int)tpitch, th, d->disp_w, d->disp_h, d->thumb_w, d->thumb_h,
-                                    d->thumb_out + (size_t)idx * d->thumb_w * d->thumb_h * 3, d->stream);
-    cudaError_t te = cudaStreamSynchronize(d->stream);
-    d->api->UnmapVideoFrame64(d->dec, tsrc);
-    if (trc != 0 || te != cudaSuccess) {
-      d->error = "thumbnail kernel failed";
-      return 0;
-    }
-    d->emitted++;
+  } else if (d->next_id >= d->n_ids || idx != d->ids[d->next_id]) {
     return 1;
-  }
-  if (d->next_id >= d->n_ids || idx != d->ids[d->next_id]) return 1;
-  if (((d->disp_w + 1) & ~1) != d->dst_w || ((d->disp_h + 1) & ~1) != d->dst_h) {
-    d->error = "clip is " + std::to_string(d->disp_w) + "x" + std::to_string(d->disp_h) + " but the surface pool is " + std::to_string(d->dst_w) +
-               "x" + std::to_string(d->dst_h);
-    return 0;
   }
   CUVIDPROCPARAMS pp;
   memset(&pp, 0, sizeof pp);
@@ -315,26 +355,9 @@ int on_display(void* user, CUVIDPARSERDISPINFO* info) {
     d->error = "cuvidMapVideoFrame64 failed with CUresult " + std::to_string(rc);
     return 0;
   }
-  const int th = d->dst_h;  // target height (even)
-  cudaError_t e = cudaSuccess;
-  while (d->next_id < d->n_ids && d->ids[d->next_id] == idx) {  // a repeated id (supersampling) fills several slots
-    uint8_t* dst = d->dst_base + (size_t)d->slots[d->next_id] * d->dst_slot_stride;
-    e = cudaMemcpy2DAsync(dst, d->dst_pitch, (const void*)src, pitch, d->dst_w, th, cudaMemcpyDeviceToDevice, d->stream);
-    if (e == cudaSuccess)
-      e = cudaMemcpy2DAsync(dst + (size_t)d->dst_luma_rows * d->dst_pitch, d->dst_pitch, (const void*)(src + (size_t)pitch * th), pitch, d->dst_w,
-                            th / 2, cudaMemcpyDeviceToDevice, d->stream);
-    if (e != cudaSuccess) break;
-    d->next_id++;
-    d->emitted++;
-  }
-  if (e == cudaSuccess) e = cudaStreamSynchronize(d->stream);  // the mapping must outlive the copy
+  const int ok = deliver(d, idx, (const uint8_t*)src, pitch);
   d->api->UnmapVideoFrame64(d->dec, src);
-  if (e != cudaSuccess) {
-    d->error = std::string("surface copy failed: ") + cudaGetErrorString(e);
-    return 0;
-  }
-  if (d->next_id >= d->n_ids) d->done = true;
-  return 1;
+  return ok;
 }
 
 int ensure_shared(cb_ctx* ctx, CuvidApi* api) {
@@ -349,6 +372,17 @@ int ensure_shared(cb_ctx* ctx, CuvidApi* api) {
   void* cuctx = nullptr;
   if (((int (*)(void**))fn)(&cuctx) != 0 || !cuctx) return cb::fail(ctx, CB_ERR_CUDA, "no current CUDA context");
   NvdecShared* s = new NvdecShared();
+  if (api->GetDecoderCaps) {
+    CUVIDDECODECAPS caps;
+    memset(&caps, 0, sizeof caps);
+    caps.eCodecType = 4, caps.eChromaFormat = 1;  // H.264 4:2:0
+    s->software = api->GetDecoderCaps(&caps) == 100;  // CUDA_ERROR_NO_DEVICE: no video engine behind this context
+  }
+  if (s->software) {
+    fprintf(stderr, "cosmos_curate_b200: the driver exposes no NVDEC engine (CUDA_ERROR_NO_DEVICE); decoding on the host with libavcodec\n");
+    ctx->nvdec = s;
+    return CB_OK;
+  }
   const int rc = api->CtxLockCreate(&s->lock, cuctx);
   if (rc != 0) {
     delete s;
@@ -408,6 +442,17 @@ int cb_mp4_cut(cb_ctx* ctx, const uint8_t* data, size_t size, int first_sample, 
   return CB_OK;
 }
 
+int cb_decode_backend(cb_ctx* ctx, int* backend) {
+  if (!ctx) return CB_ERR_ARG;
+  if (!backend) return cb::fail(ctx, CB_ERR_ARG, "decode_backend: null argument");
+  CuvidApi* api = load_cuvid();
+  if (!api->error.empty()) return cb::fail(ctx, CB_ERR_NVDEC, "%s", api->error.c_str());
+  const int rc = ensure_shared(ctx, api);
+  if (rc) return rc;
+  *backend = ((NvdecShared*)ctx->nvdec)->software ? CB_DECODE_BACKEND_LIBAVCODEC : CB_DECODE_BACKEND_NVDEC;
+  return CB_OK;
+}
+
 int cb_decoder_create(cb_ctx* ctx, cb_decoder** out) {
   if (!ctx) return CB_ERR_ARG;
   if (!out) return cb::fail(ctx, CB_ERR_ARG, "decoder_create: null argument");
@@ -417,8 +462,14 @@ int cb_decoder_create(cb_ctx* ctx, cb_decoder** out) {
   int rc = ensure_shared(ctx, api);
   if (rc) return rc;
   CB_CUDA(ctx, cudaSetDevice(ctx->device));  // the session's stream must live on this context's device, whatever thread creates it
+  const bool software = ((NvdecShared*)ctx->nvdec)->software;
+  if (software) {
+    const std::string why = cb::swdec_available();
+    if (!why.empty()) return cb::fail(ctx, CB_ERR_NVDEC, "the driver exposes no NVDEC engine (CUDA_ERROR_NO_DEVICE) and host decode is unavailable: %s", why.c_str());
+  }
   cb_decoder* d = new cb_decoder();
   d->ctx = ctx, d->api = api;
+  d->software = software;
   // highest priority: the post-processing kernel cuvidMapVideoFrame launches and the two surface copies are tiny, and the
   // decode surface is only handed back to NVDEC once they are done - they must not queue behind the tower's persistent CTAs
   int prio_lo = 0, prio_hi = 0;
@@ -435,6 +486,8 @@ void cb_decoder_destroy(cb_decoder* d) {
   if (!d) return;
   cudaSetDevice(d->ctx->device);
   if (d->dec) d->api->DestroyDecoder(d->dec);
+  cb::swdec_destroy(d->sw);
+  if (d->sw_dev) cudaFree(d->sw_dev);
   if (d->stream) cudaStreamDestroy(d->stream);
   delete d;
 }
@@ -496,7 +549,10 @@ int cb_decoder_decode_ex(cb_decoder* d, const uint8_t* data, size_t size, const 
   return run_parser(d, data, size, t, stats, d->discard ? 0 : n_ids, flags);
 }
 
+static int run_software(cb_decoder* d, const uint8_t* data, size_t size, const cb::Mp4Track& t, cb_decode_stats* stats, int expect, int flags);
+
 static int run_parser(cb_decoder* d, const uint8_t* data, size_t size, const cb::Mp4Track& t, cb_decode_stats* stats, int expect, int flags) {
+  if (d->software) return run_software(d, data, size, t, stats, expect, flags);
   cb_ctx* ctx = d->ctx;
   CUVIDPARSERPARAMS pp;
   memset(&pp, 0, sizeof pp);
@@ -567,6 +623,114 @@ static int run_parser(cb_decoder* d, const uint8_t* data, size_t size, const cb:
     stats->coded_width = (int)d->coded_w, stats->coded_height = (int)d->coded_h, stats->width = d->disp_w, stats->height = d->disp_h;
   }
   if (failed) return cb::fail(ctx, CB_ERR_NVDEC, "decode: %s", d->error.empty() ? ("cuvidParseVideoData CUresult " + std::to_string(rc)).c_str() : d->error.c_str());
+  if (d->emitted != expect) return cb::fail(ctx, CB_ERR_NVDEC, "decode: stream ended after %d displayed frames, %d of %d sampled frames delivered", d->display_index, d->emitted, expect);
+  return CB_OK;
+}
+
+// The same walk over the samples as run_parser (sync-sample seeks included), decoded by libavcodec on the host.  Every packet
+// carries its sample index as pts, and a picture's display index is the rank of that sample's composition time, exactly as
+// on_display maps NVDEC's timestamps; each wanted picture is staged as NV12 in device memory and delivered like a mapped
+// NVDEC surface.
+static int run_software(cb_decoder* d, const uint8_t* data, size_t size, const cb::Mp4Track& t, cb_decode_stats* stats, int expect, int flags) {
+  cb_ctx* ctx = d->ctx;
+  std::string err;
+  if (!d->sw || d->sw_codec != t.codec || d->sw_low_delay != !t.has_ctts) {
+    cb::swdec_destroy(d->sw);
+    d->sw = cb::swdec_create(t.codec, !t.has_ctts, &err);
+    if (!d->sw) return cb::fail(ctx, CB_ERR_NVDEC, "decode: %s", err.c_str());
+    d->sw_codec = t.codec, d->sw_low_delay = !t.has_ctts;
+  }
+  const size_t n = t.size.size();
+  {
+    std::vector<int32_t> order(n);
+    for (size_t i = 0; i < n; ++i) order[i] = (int32_t)i;
+    std::stable_sort(order.begin(), order.end(), [&](int32_t a, int32_t b) { return t.pts[a] < t.pts[b]; });
+    d->rank.assign(n, 0);
+    for (size_t r = 0; r < n; ++r) d->rank[order[r]] = (int32_t)r;
+  }
+  auto on_picture = [&](const cb::SwPicture& p) -> bool {
+    if (d->done) return true;
+    d->display_index++;
+    d->disp_w = p.width, d->disp_h = p.height, d->coded_w = 0, d->coded_h = 0;  // libavcodec does not report the coded size
+    if (d->discard) return true;
+    if (p.pts < 0 || p.pts >= (int64_t)n) {
+      d->error = "decoder returned an unknown picture timestamp";
+      return false;
+    }
+    const int idx = d->rank[(size_t)p.pts];
+    if (d->thumb_out) {
+      if (idx >= d->thumb_cap) {
+        d->done = true;
+        return true;
+      }
+    } else if (d->next_id >= d->n_ids || idx != d->ids[d->next_id]) {
+      return true;
+    }
+    const int w2 = (p.width + 1) & ~1, h2 = (p.height + 1) & ~1, cw = (p.width + 1) / 2, ch = (p.height + 1) / 2;
+    const size_t pitch = (size_t)w2, bytes = pitch * h2 * 3 / 2;
+    d->sw_host.assign(bytes, 0);
+    for (int y = 0; y < h2; ++y) memcpy(&d->sw_host[y * pitch], p.plane[0] + (size_t)std::min(y, p.height - 1) * p.pitch[0], p.width);
+    for (int y = 0; y < ch; ++y) {
+      uint8_t* row = &d->sw_host[(h2 + y) * pitch];
+      const uint8_t *u = p.plane[1] + (size_t)y * p.pitch[1], *v = p.plane[2] + (size_t)y * p.pitch[2];
+      for (int x = 0; x < cw; ++x) row[2 * x] = u[x], row[2 * x + 1] = v[x];
+    }
+    if (d->sw_dev_bytes < bytes) {
+      if (d->sw_dev) cudaFree(d->sw_dev);
+      d->sw_dev = nullptr, d->sw_dev_bytes = 0;
+      if (cudaMalloc(&d->sw_dev, bytes) != cudaSuccess) {
+        d->error = "staging surface allocation failed";
+        return false;
+      }
+      d->sw_dev_bytes = bytes;
+    }
+    if (cudaMemcpyAsync(d->sw_dev, d->sw_host.data(), bytes, cudaMemcpyHostToDevice, d->stream) != cudaSuccess) {
+      d->error = "staging surface upload failed";
+      return false;
+    }
+    return deliver(d, idx, d->sw_dev, pitch) != 0;
+  };
+  bool failed = false;
+  auto decode = [&](const uint8_t* buf, size_t len, int64_t pts) {
+    if (!cb::swdec_decode(d->sw, buf, len, pts, on_picture, &err)) failed = true;
+  };
+  auto feed = [&](size_t i) {
+    d->scratch.clear();
+    if (i == 0 || t.sync[i]) d->scratch.insert(d->scratch.end(), t.param_sets_annexb.begin(), t.param_sets_annexb.end());
+    if (!cb::mp4_sample_annexb(data, size, t, i, &d->scratch)) {
+      d->error = "malformed sample " + std::to_string(i);
+      failed = true;
+      return;
+    }
+    d->decoded++;
+    decode(d->scratch.data(), d->scratch.size(), (int64_t)i);
+  };
+  size_t pos = 0;
+  const bool seek = (flags & CB_DECODE_SEEK_SYNC) != 0 && !t.has_ctts && !d->thumb_out && !d->discard && d->n_ids > 0;
+  if (seek) {
+    for (int k = 0; k < d->n_ids && !failed && !d->done; ++k) {
+      const size_t j = (size_t)d->ids[k];
+      if (j < pos) continue;  // repeated id, already delivered
+      size_t gsync = j;
+      while (gsync > pos && !t.sync[gsync]) --gsync;
+      if (gsync > pos && t.sync[gsync]) {
+        if (pos > 0) decode(nullptr, 0, 0);
+        pos = gsync;
+      }
+      for (; pos <= j && !failed && !d->done; ++pos) feed(pos);
+    }
+  }
+  for (; pos < n && !d->done && !failed; ++pos) feed(pos);
+  if (!failed) decode(nullptr, 0, 0);  // queued pictures out; the session is ready for the next clip
+  if (stats) {
+    stats->frames_decoded = d->decoded, stats->frames_emitted = d->emitted;
+    stats->coded_width = (int)d->coded_w, stats->coded_height = (int)d->coded_h, stats->width = d->disp_w, stats->height = d->disp_h;
+  }
+  if (failed) {
+    cb::swdec_destroy(d->sw);  // state after a failure is unknown: the next call starts a fresh session
+    d->sw = nullptr;
+    return cb::fail(ctx, CB_ERR_NVDEC, "decode: %s", d->error.empty() ? err.c_str() : d->error.c_str());
+  }
   if (d->emitted != expect) return cb::fail(ctx, CB_ERR_NVDEC, "decode: stream ended after %d displayed frames, %d of %d sampled frames delivered", d->display_index, d->emitted, expect);
   return CB_OK;
 }

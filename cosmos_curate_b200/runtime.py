@@ -59,6 +59,12 @@ class Context:
         except Exception:  # noqa: BLE001
             pass
 
+    def decode_backend(self) -> str:
+        """"nvdec", or "libavcodec" where the driver exposes no NVDEC engine to this process (cb_decode_backend)."""
+        b = C.c_int()
+        check(self.lib.cb_decode_backend(self.h, C.byref(b)), "cb_decode_backend", self.h)
+        return _lib.DECODE_BACKENDS[b.value]
+
     def launch_count(self) -> int:
         return int(self.lib.cb_launch_count(self.h))
 
@@ -353,10 +359,17 @@ def mp4_index(data, ctx: Context | None = None) -> dict:
 
 
 class Decoder:
-    """One NVDEC session (cb_decoder_*).  Not thread-safe: use one per host thread."""
+    """One decode session (cb_decoder_*): NVDEC, or libavcodec on the host where the driver exposes no NVDEC engine
+    (`backend`, cb_decode_backend).  Not thread-safe: use one per host thread."""
 
     def __init__(self, ctx: Context):
         self.ctx, self.lib = ctx, ctx.lib
+        self.backend = ctx.decode_backend()
+        if self.backend == "libavcodec":
+            try:
+                import cv2  # noqa: F401 - maps opencv-python's libavcodec (and its dependencies) for the host decoder to find
+            except ImportError:
+                pass  # $CURATE_B200_LIBAVCODEC or a system libavcodec, else cb_decoder_create says what is missing
         h = C.c_void_p()
         check(self.lib.cb_decoder_create(ctx.h, C.byref(h)), "cb_decoder_create", ctx.h)
         self.h = h
@@ -386,7 +399,7 @@ class Decoder:
         check(self.lib.cb_decoder_decode_ex(self.h, buf.ctypes.data, buf.size, ids.ctypes.data_as(C.POINTER(C.c_int32)), len(ids),
                                             C.byref(pool.desc), slots.ctypes.data_as(C.POINTER(C.c_int32)), flags, C.byref(st)),
               "cb_decoder_decode", self.ctx.h)  # fmt: skip
-        return {"frames_decoded": st.frames_decoded, "frames_emitted": st.frames_emitted, "coded": (st.coded_width, st.coded_height),
+        return {"frames_decoded": st.frames_decoded, "frames_emitted": st.frames_emitted, "backend": self.backend, "coded": (st.coded_width, st.coded_height),
                 "size": (st.width, st.height)}  # fmt: skip
 
 

@@ -4,7 +4,8 @@ ClipFrameExtractionStage  (clip_frame_extraction_stages.py:43-192): fills `clip.
     keyed by FrameExtractionSignature strings, so UNMODIFIED downstream stages keep working.  Only the sampled frames
     are colour-converted (cb_nv12_to_rgb) and copied to the host.  The fused NvdecClipAestheticStage avoids even that.
 VideoFrameExtractionStage (frame_extraction_stages.py:71-204): whole video -> uint8 [n,27,48,3] in `video.frame_array`
-    (the TransNetV2 input) through NVDEC + the fused NV12->RGB+bilinear kernel; no temp file, no CPU fallback
+    (the TransNetV2 input) through cb_decoder (NVDEC; libavcodec where the driver exposes no NVDEC engine, cb_decode_backend) + the
+    fused NV12->RGB+bilinear kernel; no temp file
     (decode failure -> video.errors["frame_extraction"], like the reference's "null" result).
 """
 
@@ -147,7 +148,7 @@ class VideoFrameExtractionStage(CuratorStage):
                  batch_size: int = 64, verbose: bool = False, log_stats: bool = False) -> None:  # fmt: skip
         super().__init__()
         if decoder_mode not in ("nvdec", "pynvc"):
-            msg = f"decoder_mode={decoder_mode!r}: this stage only decodes on NVDEC (no CPU fallback on the B200 path)"
+            msg = f"decoder_mode={decoder_mode!r}: this stage decodes through cb_decoder only (NVDEC, or libavcodec where the driver exposes no NVDEC engine)"
             raise ValueError(msg)
         self.output_hw, self.decoder_mode = output_hw, decoder_mode
         self._num_gpus, self._batch, self._verbose, self._log_stats = num_gpus_per_worker, batch_size, verbose, log_stats

@@ -290,6 +290,7 @@ class NvdecClipAestheticStage(CuratorStage):
         if batches:
             finalize(len(batches) - 1)
         self.last_call_stats = {"frames_decoded": decoded, "batches": len(batches), "nvdec_sessions": self._num_decoders,
+                                "decode_backend": self._decode_pool.ctx.decode_backend(),
                                 "numa_node": self._decode_pool.numa_node, "pinned_cpus": len(self._decode_pool.cpus)}  # fmt: skip
 
     # ---- stage entry -----------------------------------------------------------------------------

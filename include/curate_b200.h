@@ -10,7 +10,8 @@
  * negative error code and never throws; cb_last_error() returns the message.  Device pointers are
  * caller-owned (torch-allocated is fine); the library owns only its context, cached tables, model
  * weights/workspace and NVDEC sessions.  `stream` is a cudaStream_t passed as void* (NULL = default).
- * There is no CPU fallback anywhere: without a CUDA device cb_init fails.
+ * Without a CUDA device cb_init fails.  Every kernel runs on the GPU; the one host-side substitute is video decode where the
+ * driver exposes no NVDEC engine to the process (cb_decode_backend), and it is reported, never silent.
  */
 #ifndef CURATE_B200_H
 #define CURATE_B200_H
@@ -188,7 +189,7 @@ typedef struct cb_mp4_info {
 
 typedef struct cb_decode_stats {
   int frames_decoded, frames_emitted;
-  int coded_width, coded_height, width, height;
+  int coded_width, coded_height, width, height; /* coded size 0 x 0 when the host decoder ran (it does not report one) */
 } cb_decode_stats;
 
 /* Index the first video track of an in-memory MP4: per-sample composition timestamps (decode order, in
@@ -206,7 +207,17 @@ int cb_mp4_index(cb_ctx* ctx, const uint8_t* data, size_t size, cb_mp4_info* inf
 int cb_mp4_cut(cb_ctx* ctx, const uint8_t* data, size_t size, int first_sample, int n_samples, uint8_t* out, size_t out_cap,
                size_t* out_size);
 
-/* One NVDEC session (parser + decoder + copy stream); use one per host thread, reuse it across clips. */
+#define CB_DECODE_BACKEND_NVDEC 0
+#define CB_DECODE_BACKEND_LIBAVCODEC 1
+/* Which decoder the sessions of this context use: NVDEC, or - when the driver exposes no NVDEC engine to the process
+ * (cuvidGetDecoderCaps -> CUDA_ERROR_NO_DEVICE, e.g. a container granted the compute capability only) - libavcodec on the
+ * host, the reference's own decoder, staging each delivered picture as NV12 in device memory.  Callers that report decode
+ * (stage stats, benchmarks) must state it.  The host decoder needs libavcodec already mapped into the process (importing
+ * cv2 maps opencv-python's copy), $CURATE_B200_LIBAVCODEC, or a system libavcodec. */
+int cb_decode_backend(cb_ctx* ctx, int* backend);
+
+/* One decode session (NVDEC parser + decoder + copy stream, or a libavcodec context, see cb_decode_backend); use one per
+ * host thread, reuse it across clips. */
 int cb_decoder_create(cb_ctx* ctx, cb_decoder** out);
 void cb_decoder_destroy(cb_decoder* dec);
 /* Decode one clip and deliver ONLY the display-order frames frame_ids[0..n_ids) (ascending; repeats allowed,

@@ -20,6 +20,8 @@ Files written (all small):
   dedup_ref.npz           the array section of SemanticDedupActor.dedup (dedup_actor.py:404-466) executed from the reference's source
                           with numpy standing in for cupy (oracle/ref_import.dedup_core) on clusters with planted duplicates
   siglip_tiny_hf.npz      transformers SiglipVisionModel tiny seeded (stand-in; not in the reference)
+  reference_cases.json    the reference's answers on the seeded cases of oracle/reference_cases.py (sampling, spans, chunking,
+                          stage-output comparator, shot logic, InternVideo2 tubes)
 
 Test infrastructure only (see oracle/__init__.py).
 """
@@ -411,6 +413,65 @@ def gen_dedup() -> None:
     print("dedup_ref.npz", {k: v.shape for k, v in out.items() if k.endswith("_maxv")})
 
 
+def gen_reference_cases() -> None:
+    """The reference's answers on the seeded cases of oracle/reference_cases.py: frame-index math, fixed-stride spans and uuids,
+    chunk sizes, the stage-output comparator, shot logic and the InternVideo2 tube formulation (tubes as sha256)."""
+    from oracle import reference_cases as R
+
+    meta: dict = {"digest": {}, "sample_closest": [], "shots": []}
+    du = ref_import.decoder_utils()
+    cases = R.timestamp_cases()
+    meta["digest"]["timestamps"] = R.digest(cases)
+    for i, c in enumerate(cases):
+        ts = c["ts"]
+        res = du.sample_closest(ts, sample_rate=c["rate"], start=ts[0], stop=ts[-1], endpoint=c["endpoint"], dedup=c["dedup"])
+        meta["sample_closest"].append({"outputs": [R.values_sha256(v) for v in res],
+                                       "find_closest": R.values_sha256(du.find_closest_indices(ts, R.closest_targets(ts)))})  # fmt: skip
+
+    f = ref_import.fixed_stride_functions()
+    cases = R.fixed_stride_cases()
+    meta["digest"]["fixed_stride"] = R.digest(cases)
+    meta["fixed_stride"] = []
+    for c in cases:
+        spans = f["_make_spans_fixed_stride"](0.0, c["end"], c["clip_len"], c["stride"], c["min_len"])
+        meta["fixed_stride"].append({"n_spans": len(spans), "spans_sha256": R.spans_sha256(spans),
+                                     "uuids_sha256": R.uuids_sha256(f["_make_clip_uuids"](c["session"], spans[:50]))})  # fmt: skip
+
+    grouping = ref_import.grouping_module()
+    cases = R.chunk_cases()
+    meta["digest"]["chunks"] = R.digest(cases)
+    meta["chunks"] = [[len(ch) for ch in grouping.split_by_chunk_size(c["spans"], c["per_chunk"] * 8, R.chunk_size)] for c in cases]
+
+    compare = ref_import.stage_compare_functions()["_compare_values"]
+    cases = R.compare_cases()
+    meta["digest"]["compare"] = R.digest(cases)
+    meta["compare"] = [[repr([R.diff_key(d) for d in compare("t", c["golden"], other, atol=c["atol"])]) for other in (c["candidate"], c["golden"])]
+                       for c in cases]  # fmt: skip
+    table = R.comparator_table()
+    meta["digest"]["comparator_table"] = R.digest(table)
+    meta["comparator_table"] = {name: repr([R.diff_key(d) for d in compare("root", g, c, atol=atol)]) for name, g, c, atol in table}
+
+    shots = ref_import.transnetv2_stage_functions()
+    cases = R.shot_cases()
+    meta["digest"]["shots"] = R.digest(cases)
+    for c in cases:
+        scenes = shots["_get_scenes"](c["track"].reshape(-1, 1), entire_scene_as_clip=c["entire"])
+        filtered = shots["_get_filtered_scenes"](scenes.copy(), min_length=c["min_len"], max_length=c["max_len"], max_length_mode=c["mode"],
+                                                 crop_length=c["crop"]) if len(scenes) else None  # fmt: skip
+        meta["shots"].append({"scenes": R.values_sha256(scenes), "dtype": scenes.dtype.str, "n_scenes": len(scenes),
+                              "filtered": None if filtered is None else R.values_sha256(filtered)})  # fmt: skip
+
+    iv2 = ref_import.internvideo2_formulator()
+    cases = R.tube_cases()
+    meta["digest"]["tubes"] = R.digest(cases)
+    meta["tubes"] = []
+    for c in cases:
+        tube = iv2._construct_frames(R.tube_frames(c), fnum=8, target_size=(c["tw"], c["th"]))
+        meta["tubes"].append({"shape": list(tube.shape), "dtype": tube.dtype.str, "sha256": R.tube_sha256(tube)})
+    (OUT / "reference_cases.json").write_text(json.dumps(meta, indent=0))
+    print("reference_cases.json")
+
+
 def main() -> None:
     assert ref_import.available(), "needs /root/reference (build container)"
     OUT.mkdir(parents=True, exist_ok=True)
@@ -423,6 +484,7 @@ def main() -> None:
     gen_dedup()
     gen_video_tube()
     gen_fixed_stride()
+    gen_reference_cases()
 
 
 if __name__ == "__main__":

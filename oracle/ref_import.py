@@ -1,8 +1,7 @@
 """Import the reference's OWN hot-path modules from /root/reference (build container only).
 
-Used by oracle/make_golden.py to produce tests/golden/* and by tests that pin the oracle when the
-checkout is present.  /root/reference does not exist on the GPU box: nothing that runs there may
-call into this module (tests skip when `available()` is False).
+Used by oracle/make_golden.py to produce tests/golden/*; the tests read those vectors and never
+call into this module, so they run without a reference checkout.
 
 Two stubs are injected, as established in SURVEY.md 8c / V2:
   * ``av``  (PyAV is not installed; only needed at import time by decoder_utils), and

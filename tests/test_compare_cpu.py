@@ -1,61 +1,29 @@
 """cosmos_curate_b200/compare.py: the reference's stage-output comparison semantics (stage_compare.py `_compare_values`), checked
-(a) against the reference functions themselves, executed from source, on a case table (build container only - /root/reference is
-absent on the GPU box) and (b) against the known answers of the reference's own tests
+(a) against the reference functions' answers on a case table (oracle/reference_cases.comparator_table, answers stored in
+tests/golden/reference_cases.json) and (b) against the known answers of the reference's own tests
 (tests/cosmos_curate/core/utils/misc/test_stage_compare.py:112-162), then used the way the reference uses it: on task lists."""
 
 from __future__ import annotations
 
+import json
 import uuid
 
-import attrs
 import numpy as np
 import pytest
+from conftest import GOLDEN
 
 from cosmos_curate_b200 import compare as C
 from cosmos_curate_b200.data_model import Clip, SplitPipeTask, Video
-from oracle import ref_import
+from oracle import reference_cases as R
 
 
-@attrs.define
-class _Leaf:
-    score: float
-    vec: np.ndarray
-    tags: dict
-
-
-def _cases():
-    a = np.arange(6, dtype=np.float32).reshape(2, 3)
-    nan = np.array([1.0, np.nan, 3.0], dtype=np.float32)
-    return [
-        ("equal", {"a": a, "b": [1, "x", (2, 3)]}, {"a": a.copy(), "b": [1, "x", (2, 3)]}, 0.0),
-        ("within", a, a + np.float32(9e-4), 1e-3),
-        ("beyond", a, a + np.float32(2e-3), 1e-3),
-        ("rtol_zero", np.array([1e6], np.float32), np.array([1e6 + 1], np.float32), 0.5),  # allclose's default rtol would pass this
-        ("unsigned", np.array([0, 255], np.uint8), np.array([1, 0], np.uint8), 0.0),
-        ("nan_match", nan, nan.copy(), 0.0),
-        ("nan_one_side", nan, np.array([1.0, 2.0, 3.0], np.float32), 0.0),
-        ("nan_plus_diff", nan, np.array([1.5, np.nan, 3.0], np.float32), 0.1),
-        ("shape", a, a.T.copy(), 1.0),
-        ("dtype_ok", a, a.astype(np.float64), 0.0),  # both ndarray: dtypes may differ
-        ("type", [1, 2], (1, 2), 0.0),
-        ("int_float", {"k": 1}, {"k": 1.0}, 0.0),
-        ("keys", {"a": 1, "b": 2}, {"a": 1, "c": 2}, 0.0),
-        ("length", [1, 2, 3], [1, 2], 0.0),
-        ("strings", np.array(["a", "b"]), np.array(["a", "c"]), 0.0),
-        ("bytes", b"abc", b"abd", 0.0),
-        ("attrs", _Leaf(1.0, a, {"x": [a]}), _Leaf(1.5, a + 1, {"x": [a * 2]}), 0.25),
-        ("nested_path", {"v": [{"w": a}]}, {"v": [{"w": a + 1}]}, 0.0),
-        ("empty", [], [], 0.0),
-    ]
-
-
-@pytest.mark.skipif(not ref_import.available(), reason="needs /root/reference (build container)")
 def test_compare_values_equals_the_reference_comparator():
-    ref = ref_import.stage_compare_functions()["_compare_values"]
-    for name, g, c, atol in _cases():
-        want = [(d.field, d.detail, d.max_diff_observed, d.shape_mismatch) for d in ref("root", g, c, atol=atol)]
-        got = [(d.field, d.detail, d.max_diff_observed, d.shape_mismatch) for d in C.compare_values("root", g, c, atol=atol)]
-        assert got == want, name
+    meta = json.loads((GOLDEN / "reference_cases.json").read_text())
+    table = R.comparator_table()
+    assert R.digest(table) == meta["digest"]["comparator_table"], "oracle/reference_cases.comparator_table changed since the golden answers were made"
+    for name, g, c, atol in table:
+        got = [R.diff_key(d) for d in C.compare_values("root", g, c, atol=atol)]
+        assert repr(got) == meta["comparator_table"][name], name
 
 
 def test_reference_known_answers():

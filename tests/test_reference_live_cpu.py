@@ -1,113 +1,76 @@
-"""Differential tests against the reference's OWN functions, imported / executed from /root/reference, on randomly generated
-inputs (hypothesis).  They run in the build container only - the GPU box has no reference checkout - and complement the committed
-golden vectors: frame-index math (decoder_utils.find_closest_indices / sample_closest), fixed-stride spans, chunk sizes and the
-stage-replay comparator must agree with the reference on inputs nobody hand-picked."""
+"""Differential tests against the reference's OWN functions on generated inputs: frame-index math (decoder_utils.find_closest_indices
+/ sample_closest), fixed-stride spans, chunk sizes, the stage-replay comparator, shot logic and the InternVideo2 tube formulation
+must agree with the reference on inputs nobody hand-picked.  The inputs are the seeded cases of oracle/reference_cases.py; the
+reference's answers on them are stored in tests/golden/reference_cases.json (`python -m oracle.make_golden` regenerates them from
+a reference checkout)."""
 
 from __future__ import annotations
 
-import numpy as np
+import json
+
 import pytest
-from hypothesis import HealthCheck, given, settings
-from hypothesis import strategies as st
+from conftest import GOLDEN
 
 from cosmos_curate_b200 import compare as C
 from cosmos_curate_b200 import sampling as S
 from cosmos_curate_b200 import spans as SP
-from oracle import ref_import
-
-pytestmark = pytest.mark.skipif(not ref_import.available(), reason="needs /root/reference (build container)")
-_cfg = settings(max_examples=150, deadline=None, suppress_health_check=[HealthCheck.too_slow])
+from oracle import reference_cases as R
 
 
-@st.composite
-def _timestamps(draw):
-    """Sorted float32 presentation times: constant or variable frame rate, optional dropped frames, optional start offset."""
-    n = draw(st.integers(2, 400))
-    fps = draw(st.sampled_from([10.0, 23.976, 24.0, 25.0, 29.97, 30.0, 50.0, 59.94, 60.0]))
-    t = np.arange(n, dtype=np.float64) / fps + draw(st.sampled_from([0.0, 0.0, 0.033, 1.5]))
-    if draw(st.booleans()):
-        t = t + np.cumsum(draw(st.lists(st.floats(0.0, 0.02), min_size=n, max_size=n)))  # variable frame rate
-    if draw(st.booleans()) and n > 10:
-        keep = np.ones(n, bool)
-        keep[draw(st.lists(st.integers(1, n - 2), max_size=n // 5))] = False  # dropped frames
-        t = t[keep]
-    return np.sort(t.astype(np.float32))
+@pytest.fixture(scope="module")
+def ref():
+    return json.loads((GOLDEN / "reference_cases.json").read_text())
 
 
-@_cfg
-@given(ts=_timestamps(), rate=st.sampled_from([0.5, 1.0, 2.0, 3.0, 4.0, 7.5, 8.0, 16.0, 30.0, 100.0]), endpoint=st.booleans(), dedup=st.booleans())
-def test_sample_closest_agrees_with_the_reference(ts, rate, endpoint, dedup):
-    du = ref_import.decoder_utils()
-    want = du.sample_closest(ts, sample_rate=rate, start=ts[0], stop=ts[-1], endpoint=endpoint, dedup=dedup)
-    got = S.sample_closest(ts, rate, start=ts[0], stop=ts[-1], endpoint=endpoint, dedup=dedup)
-    for g, w in zip(got, want):
-        assert np.array_equal(np.asarray(g), np.asarray(w))
-    dst = np.linspace(float(ts[0]) - 0.3, float(ts[-1]) + 0.3, 57).astype(np.float32)
-    assert np.array_equal(S.find_closest_indices(ts, dst), du.find_closest_indices(ts, dst))
+def _cases(ref, name: str, cases: list) -> list:
+    assert R.digest(cases) == ref["digest"][name], f"oracle/reference_cases.py no longer generates the {name} cases the golden answers were made for"
+    return cases
 
 
-@_cfg
-@given(end=st.floats(0.0, 400.0), clip_len=st.floats(0.1, 60.0), stride=st.floats(0.05, 90.0), min_len=st.floats(0.0, 30.0), session=st.text(min_size=0, max_size=12))
-def test_fixed_stride_spans_and_uuids_agree_with_the_reference(end, clip_len, stride, min_len, session):
-    f = ref_import.fixed_stride_functions()
-    want = f["_make_spans_fixed_stride"](0.0, end, clip_len, stride, min_len)
-    got = SP.make_spans_fixed_stride(0.0, end, clip_len, stride, min_len)
-    assert [(float.hex(a), float.hex(b)) for a, b in got] == [(float.hex(a), float.hex(b)) for a, b in want]
-    assert SP.make_clip_uuids(session, got[:50]) == f["_make_clip_uuids"](session, want[:50])
+def test_sample_closest_agrees_with_the_reference(ref):
+    for i, (c, want) in enumerate(zip(_cases(ref, "timestamps", R.timestamp_cases()), ref["sample_closest"], strict=True)):
+        ts = c["ts"]
+        got = S.sample_closest(ts, c["rate"], start=ts[0], stop=ts[-1], endpoint=c["endpoint"], dedup=c["dedup"])
+        assert [R.values_sha256(g) for g in got] == want["outputs"], i
+        assert R.values_sha256(S.find_closest_indices(ts, R.closest_targets(ts))) == want["find_closest"], i
 
 
-@_cfg
-@given(durs=st.lists(st.floats(0.0, 40.0), max_size=120), per_chunk=st.integers(1, 40))
-def test_chunk_sizes_agree_with_the_reference(durs, per_chunk):
-    spans = [(float(i), float(i) + d) for i, d in enumerate(durs)]
-    size = lambda s: int(s[1] - s[0])  # noqa: E731
-    want = [len(c) for c in ref_import.grouping_module().split_by_chunk_size(spans, per_chunk * 8, size)]
-    assert [len(c) for c in SP.split_by_chunk_size(spans, per_chunk * 8, size)] == want
+def test_fixed_stride_spans_and_uuids_agree_with_the_reference(ref):
+    for c, want in zip(_cases(ref, "fixed_stride", R.fixed_stride_cases()), ref["fixed_stride"], strict=True):
+        got = SP.make_spans_fixed_stride(0.0, c["end"], c["clip_len"], c["stride"], c["min_len"])
+        assert len(got) == want["n_spans"] and R.spans_sha256(got) == want["spans_sha256"]
+        assert R.uuids_sha256(SP.make_clip_uuids(c["session"], got[:50])) == want["uuids_sha256"]
 
 
-_leaf = st.one_of(st.integers(-5, 5), st.floats(-2, 2, allow_nan=False), st.text(max_size=3), st.booleans(), st.none(),
-                  st.builds(lambda v, d: np.array(v, dtype=d), st.lists(st.one_of(st.floats(-3, 3, width=32), st.just(float("nan"))), max_size=5), st.sampled_from(["float32", "float64"])),
-                  st.builds(lambda v: np.array(v, dtype=np.uint8), st.lists(st.integers(0, 255), max_size=5)))  # fmt: skip
-_tree = st.recursive(_leaf, lambda kids: st.one_of(st.lists(kids, max_size=4), st.tuples(kids, kids), st.dictionaries(st.sampled_from(["a", "b", "c", 1]), kids, max_size=3)), max_leaves=12)
+def test_chunk_sizes_agree_with_the_reference(ref):
+    for c, want in zip(_cases(ref, "chunks", R.chunk_cases()), ref["chunks"], strict=True):
+        assert [len(ch) for ch in SP.split_by_chunk_size(c["spans"], c["per_chunk"] * 8, R.chunk_size)] == want
 
 
-@_cfg
-@given(golden=_tree, candidate=_tree, atol=st.sampled_from([0.0, 1e-3, 0.5, 2.0]))
-def test_compare_values_agrees_with_the_reference(golden, candidate, atol):
-    ref = ref_import.stage_compare_functions()["_compare_values"]
-    key = lambda d: (d.field, d.detail, d.max_diff_observed, d.shape_mismatch)  # noqa: E731
-    for g, c in ((golden, candidate), (golden, golden)):
-        want, got = [key(d) for d in ref("t", g, c, atol=atol)], [key(d) for d in C.compare_values("t", g, c, atol=atol)]
-        assert repr(got) == repr(want)  # repr: NaN-carrying details compare equal as text
+def test_compare_values_agrees_with_the_reference(ref):
+    for c, want in zip(_cases(ref, "compare", R.compare_cases()), ref["compare"], strict=True):
+        for other, w in zip((c["candidate"], c["golden"]), want, strict=True):
+            got = [R.diff_key(d) for d in C.compare_values("t", c["golden"], other, atol=c["atol"])]
+            assert repr(got) == w  # repr: NaN-carrying details compare equal as text
 
 
-@_cfg
-@given(track=st.lists(st.sampled_from([0, 0, 0, 0, 1]), min_size=1, max_size=600), entire=st.booleans(), min_len=st.one_of(st.none(), st.integers(1, 80)),
-       max_len=st.one_of(st.none(), st.integers(1, 200)), mode=st.sampled_from(["truncate", "stride"]), crop=st.one_of(st.none(), st.integers(0, 20)))
-def test_shot_logic_agrees_with_the_reference(track, entire, min_len, max_len, mode, crop):
+def test_shot_logic_agrees_with_the_reference(ref):
     """0/1 transition tracks -> scenes -> filtered scenes: transnetv2_extraction_stages._get_scenes / _get_filtered_scenes."""
     from cosmos_curate_b200 import shots
 
-    f = ref_import.transnetv2_stage_functions()
-    pred = np.array(track, dtype=np.uint8).reshape(-1, 1)
-    want = f["_get_scenes"](pred, entire_scene_as_clip=entire)
-    got = shots.scenes_from_predictions(pred, entire_scene_as_clip=entire)
-    assert np.array_equal(got, want) and got.dtype == want.dtype
-    if len(want):
-        want_f = f["_get_filtered_scenes"](want.copy(), min_length=min_len, max_length=max_len, max_length_mode=mode, crop_length=crop)
-        got_f = shots.filter_scenes(got.copy(), min_length=min_len, max_length=max_len, max_length_mode=mode, crop_length=crop)
-        assert np.array_equal(got_f, want_f)
+    for i, (c, want) in enumerate(zip(_cases(ref, "shots", R.shot_cases()), ref["shots"], strict=True)):
+        got = shots.scenes_from_predictions(c["track"].reshape(-1, 1), entire_scene_as_clip=c["entire"])
+        assert len(got) == want["n_scenes"] and R.values_sha256(got) == want["scenes"] and got.dtype.str == want["dtype"], i
+        if len(got):
+            got_f = shots.filter_scenes(got.copy(), min_length=c["min_len"], max_length=c["max_len"], max_length_mode=c["mode"], crop_length=c["crop"])
+            assert R.values_sha256(got_f) == want["filtered"], i
 
 
-@settings(max_examples=60, deadline=None, suppress_health_check=[HealthCheck.too_slow])
-@given(h=st.integers(1, 260), w=st.integers(1, 260), th=st.integers(1, 72), tw=st.integers(1, 72), n=st.integers(8, 19), seed=st.integers(0, 2**31 - 1))
-def test_video_tube_oracle_agrees_with_the_reference_formulation(h, w, th, tw, n, seed):
+def test_video_tube_oracle_agrees_with_the_reference_formulation(ref):
     """oracle/video_tube.py vs InternVideo2MultiModality._construct_frames (cv2.resize + numpy) on arbitrary sizes, every float32 bit:
     up- and down-scaling, 1-pixel sources and targets, the exact-2x INTER_AREA reroute, the copy for equal sizes."""
     from oracle import video_tube as T
 
-    rng = np.random.default_rng(seed)
-    frames = [rng.integers(0, 256, size=(h, w, 3), dtype=np.uint8) for _ in range(n)]
-    want = ref_import.internvideo2_formulator()._construct_frames(frames, fnum=8, target_size=(tw, th))
-    got = T.construct_frames(frames, fnum=8, target_size=(tw, th))
-    assert got.shape == want.shape and np.array_equal(got, want)
+    for c, want in zip(_cases(ref, "tubes", R.tube_cases()), ref["tubes"], strict=True):
+        got = T.construct_frames(R.tube_frames(c), fnum=8, target_size=(c["tw"], c["th"]))
+        assert list(got.shape) == want["shape"] and got.dtype.str == want["dtype"] and R.tube_sha256(got) == want["sha256"], c

@@ -25,8 +25,8 @@ _DECODE = textwrap.dedent(
     w, h, fps, secs, deblock = int(sys.argv[2]), int(sys.argv[3]), 30, float(sys.argv[4]), sys.argv[5] == "1"
     mp4, info = S.make_coded_clip(w, h, fps, secs, seed=int(sys.argv[6]), bitrate=float(sys.argv[7]), deblock=deblock,
                                   ac_density=0.25 if deblock else 0.0, return_info=True)
-    open("/tmp/_cb_coded.mp4", "wb").write(mp4)
-    cap = cv2.VideoCapture("/tmp/_cb_coded.mp4")
+    open(sys.argv[8], "wb").write(mp4)
+    cap = cv2.VideoCapture(sys.argv[8])
     cap.set(cv2.CAP_PROP_CONVERT_RGB, 0)
     pcm = info["pcm"][:256].reshape(16, 16)
     rows = h - (h // 16) * 16 or 16   # visible rows of the last macroblock row
@@ -50,8 +50,8 @@ _DECODE = textwrap.dedent(
 )
 
 
-def _run(w, h, secs, deblock, seed, bitrate):
-    r = subprocess.run([sys.executable, "-c", _DECODE, str(ROOT), str(w), str(h), str(secs), "1" if deblock else "0", str(seed), str(bitrate)],
+def _run(w, h, secs, deblock, seed, bitrate, tmp_path):
+    r = subprocess.run([sys.executable, "-c", _DECODE, str(ROOT), str(w), str(h), str(secs), "1" if deblock else "0", str(seed), str(bitrate), str(tmp_path / "coded.mp4")],
                        capture_output=True, text=True, timeout=600)  # fmt: skip
     assert r.returncode == 0, r.stderr[-2000:]
     errs = [line for line in r.stderr.splitlines() if "OPENCV:FFMPEG" in line]
@@ -60,15 +60,15 @@ def _run(w, h, secs, deblock, seed, bitrate):
     return json.loads(r.stdout.strip().splitlines()[-1]), errs
 
 
-def test_coded_clip_is_conforming_and_closed_loop_exact():
-    out, errs = _run(640, 368, 3.0, False, 4, 1.0e6)
+def test_coded_clip_is_conforming_and_closed_loop_exact(tmp_path):
+    out, errs = _run(640, 368, 3.0, False, 4, 1.0e6, tmp_path)
     assert errs == []
     assert out["frames"] == 90 and out["sentinel_ok"] == 90
     assert out["idr_mismatch"] == [0, 0, 0]  # deblocking off, DC only: the IDR luma IS the mosaic
 
 
-def test_coded_clip_1080p_bitrate_and_deblocking():
-    out, errs = _run(1920, 1080, 2.0, True, 9, 4.0e6)
+def test_coded_clip_1080p_bitrate_and_deblocking(tmp_path):
+    out, errs = _run(1920, 1080, 2.0, True, 9, 4.0e6, tmp_path)
     assert errs == []
     assert out["frames"] == 60 and out["sentinel_ok"] == 60  # 1080 = 67.5 macroblock rows: the sentinel is half visible
     assert abs(out["bitrate"] - 4.0e6) / 4.0e6 < 0.12, out  # the reference's transcode default (decoder_utils.py:43)
