@@ -1,15 +1,23 @@
-// Second-generation tcgen05 attention for head_dim 64 / 129..257 tokens: same tiling as attention_tc.cu (two 128-row query
-// tiles x one 256-key tile per (image, head), S in TMEM, V as MN-major B operand, token 256 folded in on SIMT), but TWO
-// threads per query row.  The first kernel gave each row to one thread; with 8 softmax warps per SM (2 per scheduler) it was
-// bound by issue slots and latency (clock64 trace in DESIGN.md), not by MUFU, TMEM or the tensor pipe.  Here 16 softmax warps
+// softmax(Q K^T / sqrt(d)) V on the tcgen05 tensor cores for the ViT-L/14 shape class: head_dim 64, 129..257 tokens.
+//
+// 257 = 2 * 128 + 1: the first 256 tokens map onto the tensor cores with no padding at all - two 128-row query tiles
+// against one 256-key tile (S = Q K^T is ONE UMMA 128x256x64 per query tile; no online softmax, every key of the row is
+// in TMEM at once) - and token 256 is folded in on the SIMT side: its key/value as one extra column per row, its query
+// row by dedicated warps.  Persistent CTAs (one per SM) loop over (image, head) pairs.  P = exp(S) goes back through
+// shared memory in the 128-byte-swizzled K-major layout of the UMMA A operand, and O += P V (M128 N64 K64 per 64-key
+// chunk) consumes V straight from its [key][dim] rows as an MN-major B operand, with no transpose pass.
+// TMEM: 512 columns = S_0 | S_1 (256 fp32 columns each); O_g reuses columns 0..63 of S_g once P has been formed from them.
+//
+// Two threads per query row.  With one thread per row (8 softmax warps per SM, 2 per scheduler) the softmax is bound by
+// issue slots and latency (clock64 trace in DESIGN.md), not by MUFU, TMEM or the tensor pipe.  Here 16 softmax warps
 // (4 per scheduler) each own 32 rows x 128 columns: the row maximum and the row sum are combined across the two half-rows
 // through shared memory (one named barrier per group each), every half-row exponentiates its own two 64-key chunks into its
 // own P buffer, and the epilogue writes 32 of the 64 output dims per thread.
 //
 // Warp roles (704 threads): 0 TMA producer, 1 MMA issuer (event loop), 2, 3, 20, 21 query row 256 on SIMT (64 keys each),
 // 4..19 softmax: group g = (w-4)/8 (query tile), half hf = ((w-4)/4)%2 (key columns hf*128..+127), TMEM lane quarter w%4.
-// The extra row used to be ONE warp (257 dot products + a 257-term weighted sum, ~8k cycles per unit): every K and V
-// buffer release waited for it, and it - not the exponentials - set the pace of the whole kernel.
+// Query row 256 is split over four warps because every K and V buffer release waits for it: on one warp (257 dot
+// products + a 257-term weighted sum, ~8k cycles per unit) it, not the exponentials, sets the pace of the whole kernel.
 #include <cstdlib>
 #include <cstring>
 
@@ -63,7 +71,9 @@ __device__ __forceinline__ void tmem_ld_wait_pin(uint32_t* r) {
                  "+r"(r[21]), "+r"(r[22]), "+r"(r[23]), "+r"(r[24]), "+r"(r[25]), "+r"(r[26]), "+r"(r[27]), "+r"(r[28]), "+r"(r[29]), "+r"(r[30]),
                  "+r"(r[31])::"memory");
 }
-__device__ __forceinline__ uint64_t umma_desc_sw128_mn(uint32_t smem_addr) {  // see attention_tc.cu
+// MN-major B operand, SW128: rows are K (keys), each row = 64 contiguous N elements (128 B); 8-row groups 1024 B apart.
+// LBO (stride between 64-element column blocks along N) is irrelevant for N = 64; both strides are set to 1024 B.
+__device__ __forceinline__ uint64_t umma_desc_sw128_mn(uint32_t smem_addr) {
   uint64_t d = 0;
   d |= (uint64_t)((smem_addr & 0x3FFFF) >> 4);
   d |= (uint64_t)(1024 >> 4) << 16;
@@ -465,7 +475,7 @@ __global__ void __launch_bounds__(kThreads, 1)
 int attention_tc2(cb_ctx* ctx, const void* qkv, void* out, int n, int tokens, int heads, int head_dim, cudaStream_t stream, bool* launched) {
   *launched = false;
   const char* sel = std::getenv("CB_ATTN_KERNEL");
-  if (sel && (std::strcmp(sel, "mma") == 0 || std::strcmp(sel, "tc1") == 0)) return CB_OK;  // A/B switches: tc1 = one thread per row, mma = mma.sync
+  if (sel && std::strcmp(sel, "mma") == 0) return CB_OK;  // force the mma.sync kernel (the reference the tests compare against)
   if (head_dim != 64 || tokens < 129 || tokens > 257) return CB_OK;
   const int hidden = heads * 64;
   CUtensorMap map, map_row;

@@ -1,6 +1,6 @@
 // Fused frame preprocess kernels (sm_100a).
 //
-//  clip_preprocess_kernel : NV12 (or RGB24) frame -> YUV->RGB u8 (OpenCV BT.601 fixed point) ->
+//  clip_preprocess_v2_kernel : NV12 (or RGB24) frame -> YUV->RGB u8 (OpenCV BT.601 or libswscale fixed point) ->
 //      antialiased bicubic resize (ATen _upsample_bicubic2d_aa arithmetic, horizontal then vertical,
 //      fp32 FMA chains in tap order) -> centre crop -> clamp/round to u8 -> (v/255 - mean)/std LUT ->
 //      fp16/bf16/fp32, NCHW or patch-major rows for the tower's patch-embed GEMM.
@@ -8,6 +8,8 @@
 //      Source strips are staged into shared memory by TMA (cp.async.bulk.tensor, mbarrier double buffer);
 //      a CTA owns one frame x one tile of output columns and walks down the source rows keeping a ring
 //      of horizontally filtered rows, so every source byte is fetched once per column tile.
+//      By default the horizontal pass runs on the tensor pipe instead (preprocess_tc.cu); this SIMT kernel takes RGB24
+//      pools, more than 40 vertical taps and the plans the tensor-pipe kernel rejects, and CB_PRE_KERNEL=2 forces it.
 //  bilinear_u8_kernel     : NV12 -> RGB -> 4-tap bilinear (half-pixel centres) -> u8 HWC (27x48 frames).
 //  nv12_to_rgb_kernel     : full-resolution NV12 -> RGB24.
 #include <cuda_bf16.h>
@@ -16,6 +18,7 @@
 #include <algorithm>
 #include <cmath>
 #include <cstdlib>
+#include <cstring>
 
 #include "common.h"
 #include "ptx.cuh"
@@ -50,11 +53,6 @@ __device__ __forceinline__ void yuv_to_rgb_sws(int y, int u, int v, int& r, int&
   g = min(max(g, 0), 255);
   b = min(max(b, 0), 255);
 }
-template <int FMT>
-__device__ __forceinline__ void yuv_to_rgb_fmt(int y, int u, int v, int& r, int& g, int& b) {
-  if (FMT == CB_FMT_NV12_SWS) yuv_to_rgb_sws(y, u, v, r, g, b);
-  else yuv_to_rgb(y, u, v, r, g, b);
-}
 __host__ __device__ __forceinline__ constexpr bool is_nv12(int fmt) { return fmt == CB_FMT_NV12 || fmt == CB_FMT_NV12_SWS; }
 
 constexpr int kThreads = 256;
@@ -74,7 +72,7 @@ struct ClipArgs {
   const float* lut;       // [3][256]
   int out_mode;           // 0 = u8 NCHW, 1 = typed NCHW, 2 = typed patch rows
   int x_align;            // source window start is aligned down to this many pixels (TMA: 16-byte aligned box start)
-  int gu;                 // v2: rows of the per-group dense weight table (>= widest 4-column union window)
+  int gu;                 // rows of the per-group dense weight table (>= widest 4-column union window)
   int dtype, patch, k_pad;
   void* out;
 };
@@ -100,166 +98,14 @@ __device__ __forceinline__ void store_typed(void* out, size_t idx, float v, int 
   else ((float*)out)[idx] = v;
 }
 
-template <int FMT>
-__global__ void __launch_bounds__(kThreads) clip_preprocess_kernel(const __grid_constant__ CUtensorMap map_a,
-                                                                     const __grid_constant__ CUtensorMap map_b, const ClipArgs a) {
-  extern __shared__ __align__(128) uint8_t smem[];
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int frame = blockIdx.y;
-  const int c0 = blockIdx.x * a.tc;
-  const int ncol = min(a.tc, a.res_out - c0);
-  const int slot = a.slots[frame];
-
-  // ---- shared memory carve-up
-  const int raw_stage = is_nv12(FMT) ? (a.swa * kSR + a.swa * (kSR / 2)) : (3 * a.swa * kSR);
-  const int swp = a.swa + 1;  // odd pitch: lanes walk rows without bank conflicts
-  const int tcp = a.tc | 1;
-  uint8_t* raw = smem;                                                  // [2][raw_stage]
-  float* rgbf = (float*)(smem + 2 * raw_stage);                         // [3][kSR][swp]
-  float* ringb = rgbf + 3 * kSR * swp;                                  // [3][ring][tcp]
-  uint16_t* obuf = (uint16_t*)(ringb + 3 * a.ring * tcp);               // patch staging [tc/patch][k_pad]
-  const int npx = (a.out_mode == 2) ? a.tc / a.patch : 0;
-  uint64_t* bars = (uint64_t*)(((uintptr_t)(obuf + npx * a.k_pad) + 7) & ~(uintptr_t)7);
-
-  // source columns this tile touches
-  const int x_lo = a.xmin[c0] & ~(a.x_align - 1);
-
-  if (tid == 0) {
-    mbar_init(&bars[0], 1);
-    mbar_init(&bars[1], 1);
-    fence_barrier_init();
-  }
-  if (a.out_mode == 2)
-    for (int i = tid; i < npx * a.k_pad; i += kThreads) obuf[i] = 0;  // zero K padding once
-  __syncthreads();
-
-  // NOTE: x_lo is a multiple of 16 pixels: a TMA box whose first byte is not 16-byte aligned in global memory
-  // faults with "illegal instruction" (measured on B200; u8 elements make this easy to hit).
-#define CB_ISSUE_STRIP(S_)                                                                                        \
-  do {                                                                                                            \
-    const int s_ = (S_);                                                                                          \
-    uint8_t* dst_ = raw + (s_ & 1) * raw_stage;                                                                   \
-    uint64_t* bar_ = &bars[s_ & 1];                                                                               \
-    const int ys_ = a.y_begin + s_ * kSR;                                                                         \
-    mbar_expect_tx(bar_, raw_stage);                                                                              \
-    if (is_nv12(FMT)) {                                                                                     \
-      tma_load_3d(dst_, &map_a, bar_, x_lo, ys_, slot);                                                           \
-      tma_load_3d(dst_ + a.swa * kSR, &map_b, bar_, x_lo, ys_ >> 1, slot);                                        \
-    } else {                                                                                                      \
-      tma_load_3d(dst_, &map_a, bar_, x_lo * 3, ys_, slot);                                                       \
-      tma_load_3d(dst_ + a.swa * kSR, &map_a, bar_, x_lo * 3 + a.swa, ys_, slot);                                 \
-      tma_load_3d(dst_ + 2 * a.swa * kSR, &map_a, bar_, x_lo * 3 + 2 * a.swa, ys_, slot);                         \
-    }                                                                                                             \
-  } while (0)
-  if (tid == 0) {
-    CB_ISSUE_STRIP(0);
-    if (a.n_strips > 1) CB_ISSUE_STRIP(1);
-  }
-
-  int next_out = 0;  // next output row to emit
-  for (int s = 0; s < a.n_strips; ++s) {
-    const int y0 = a.y_begin + s * kSR;
-    const uint8_t* rs = raw + (s & 1) * raw_stage;
-    mbar_wait(&bars[s & 1], (s >> 1) & 1);
-
-    // ---- phase 1: colour convert the strip to planar fp32 RGB (values are exact u8 integers)
-    if (is_nv12(FMT)) {
-      const int half_w = a.swa >> 1;
-      const uint8_t* ry = rs;
-      const uint8_t* ruv = rs + a.swa * kSR;
-      for (int i = tid; i < kSR * half_w; i += kThreads) {
-        const int r = i / half_w, x = (i - r * half_w) * 2;
-        const uchar2 yy = *(const uchar2*)(ry + r * a.swa + x);
-        const uchar2 uv = *(const uchar2*)(ruv + (r >> 1) * a.swa + x);
-        int R, G, B;
-        float* p = rgbf + r * swp + x;
-        yuv_to_rgb_fmt<FMT>(yy.x, uv.x, uv.y, R, G, B);
-        p[0] = (float)R, p[kSR * swp] = (float)G, p[2 * kSR * swp] = (float)B;
-        yuv_to_rgb_fmt<FMT>(yy.y, uv.x, uv.y, R, G, B);
-        p[1] = (float)R, p[kSR * swp + 1] = (float)G, p[2 * kSR * swp + 1] = (float)B;
-      }
-    } else {
-      for (int i = tid; i < kSR * a.swa; i += kThreads) {
-        const int r = i / a.swa, x = i - r * a.swa;
-#pragma unroll
-        for (int ch = 0; ch < 3; ++ch) {
-          const int b = 3 * x + ch;
-          const int blk = b / a.swa, within = b - blk * a.swa;
-          rgbf[(ch * kSR + r) * swp + x] = (float)rs[(blk * kSR + r) * a.swa + within];
-        }
-      }
-    }
-    __syncthreads();
-    if (tid == 0 && s + 2 < a.n_strips) {
-      fence_proxy_async();  // generic-proxy reads of this stage are done; hand it back to the TMA
-      CB_ISSUE_STRIP(s + 2);
-    }
-
-    // ---- phase 2: horizontal filter; lane = source row of the strip, (column, channel) uniform per warp
-    for (int item = warp; item < ncol * 3; item += kThreads / 32) {
-      const int c = item / 3, ch = item - c * 3;
-      const int xs = a.xsize[c0 + c];
-      const float* w = a.wx + (size_t)(c0 + c) * a.tx;
-      const float* src = rgbf + (ch * kSR + lane) * swp + (a.xmin[c0 + c] - x_lo);
-      float acc = src[0] * __ldg(w);
-      for (int j = 1; j < xs; ++j) acc = fmaf(src[j], __ldg(w + j), acc);
-      ringb[(ch * a.ring + ((y0 + lane) & (a.ring - 1))) * tcp + c] = acc;
-    }
-    __syncthreads();
-
-    // ---- phase 3: emit every output row whose vertical window is now complete
-    int last = next_out;
-    const bool final_strip = (s == a.n_strips - 1);
-    while (last < a.res_out && (final_strip || a.ymin[last] + a.ysize[last] <= y0 + kSR)) ++last;
-    for (int yo = next_out; yo < last; ++yo) {
-      const int ym = a.ymin[yo], ys = a.ysize[yo];
-      const float* w = a.wy + (size_t)yo * a.ty;
-      for (int item = tid; item < ncol * 3; item += kThreads) {
-        const int ch = item / ncol, c = item - ch * ncol;
-        const float* rb = ringb + (size_t)ch * a.ring * tcp + c;
-        float acc = rb[(ym & (a.ring - 1)) * tcp] * __ldg(w);
-        for (int k = 1; k < ys; ++k) acc = fmaf(rb[((ym + k) & (a.ring - 1)) * tcp], __ldg(w + k), acc);
-        acc = fminf(fmaxf(acc, 0.f), 255.f);
-        const int v = __float2int_rn(acc);  // round half to even == torch.round
-        const int x = c0 + c;
-        if (a.out_mode == 0) {
-          ((uint8_t*)a.out)[(((size_t)frame * 3 + ch) * a.res + yo) * a.res + x] = (uint8_t)v;
-        } else {
-          const float f = a.lut[ch * 256 + v];
-          if (a.out_mode == 1) {
-            store_typed(a.out, (((size_t)frame * 3 + ch) * a.res + yo) * a.res + x, f, a.dtype);
-          } else {
-            const int ip = c / a.patch, px = c - ip * a.patch, py = yo % a.patch;
-            const uint16_t bits = (a.dtype == CB_DT_F16) ? __half_as_ushort(__float2half_rn(f))
-                                                         : __bfloat16_as_ushort(__float2bfloat16_rn(f));
-            obuf[ip * a.k_pad + (ch * a.patch + py) * a.patch + px] = bits;
-          }
-        }
-      }
-      if (a.out_mode == 2 && (yo % a.patch) == a.patch - 1) {  // a row of patches is complete: 128-bit stores
-        __syncthreads();
-        const int g = a.res / a.patch, prow = yo / a.patch, vec = a.k_pad >> 3;
-        const int np = ncol / a.patch;
-        for (int i = tid; i < np * vec; i += kThreads) {
-          const int ip = i / vec, q = i - ip * vec;
-          uint4* dst = (uint4*)((uint16_t*)a.out + ((size_t)frame * g * g + (size_t)prow * g + (c0 / a.patch + ip)) * a.k_pad);
-          dst[q] = ((const uint4*)(obuf + ip * a.k_pad))[q];
-        }
-        __syncthreads();
-      }
-    }
-    next_out = last;
-  }
-}
-
-
-// ------------------------------------------------------------------------------------------------ v2
-// Same data flow as clip_preprocess_kernel, re-tiled so the horizontal pass stops being shared-memory bound:
+// ------------------------------------------------------------------------------------------------
+// Tiled so that the horizontal pass is not shared-memory bound:
 //   * output columns are processed in groups of 4 adjacent columns; their tap windows overlap by ~75 %, so one
 //     lane (= one source row) walks the UNION window once, loading each pixel once (3 x LDS.32) and applying it to
-//     the 4 columns with a dense, zero-padded weight row fetched as one broadcast LDS.128: 12 FMAs per 4 loads
-//     instead of 1 FMA per 2 loads.  fma(x, 0, acc) == acc, so the result is bit-identical to the tap-order chain.
-//   * colour conversion uses add-min-relu (DPX) instead of separate add / shift / clamp chains;
+//     the 4 columns with a dense, zero-padded weight row fetched as one broadcast LDS.128: 12 FMAs per 4 loads, where
+//     a lane walking one column's own window does 1 FMA per 2 loads.  fma(x, 0, acc) == acc, so the result is
+//     bit-identical to the tap-order chain.
+//   * colour conversion clamps with add-min-relu (DPX) instead of separate add / shift / clamp chains;
 //   * all output rows that became ready in a strip are emitted in one parallel sweep.
 template <int FMT>
 __global__ void __launch_bounds__(kThreads, 2) clip_preprocess_v2_kernel(const __grid_constant__ CUtensorMap map_a,
@@ -312,7 +158,9 @@ __global__ void __launch_bounds__(kThreads, 2) clip_preprocess_v2_kernel(const _
   }
   __syncthreads();
 
-#define CB_ISSUE_STRIP2(S_)                                                                                       \
+  // NOTE: x_lo is a multiple of 16 pixels: a TMA box whose first byte is not 16-byte aligned in global memory
+  // faults with "illegal instruction" (measured on B200; u8 elements make this easy to hit).
+#define CB_ISSUE_STRIP(S_)                                                                                        \
   do {                                                                                                            \
     const int s_ = (S_);                                                                                          \
     uint8_t* dst_ = raw + (s_ & 1) * raw_stage;                                                                   \
@@ -329,8 +177,8 @@ __global__ void __launch_bounds__(kThreads, 2) clip_preprocess_v2_kernel(const _
     }                                                                                                             \
   } while (0)
   if (tid == 0) {
-    CB_ISSUE_STRIP2(0);
-    if (a.n_strips > 1) CB_ISSUE_STRIP2(1);
+    CB_ISSUE_STRIP(0);
+    if (a.n_strips > 1) CB_ISSUE_STRIP(1);
   }
 
   int next_out = 0;
@@ -399,7 +247,7 @@ __global__ void __launch_bounds__(kThreads, 2) clip_preprocess_v2_kernel(const _
     __syncthreads();
     if (tid == 0 && s + 2 < a.n_strips) {
       fence_proxy_async();
-      CB_ISSUE_STRIP2(s + 2);
+      CB_ISSUE_STRIP(s + 2);
     }
 
     // ---- phase 2: horizontal filter, 4 columns x 3 channels per lane (lane = source row)
@@ -887,7 +735,7 @@ int run_clip_preprocess(cb_ctx* ctx, const cb_surface_pool* pool, const int32_t*
     a.tc = out_mode == 2 ? layout_patch * std::max(1, 16 / layout_patch) : 16;
   }
   a.swa = (span + 15) & ~15;
-  // v2: widest union window of any group of 4 adjacent output columns
+  // widest union window of any group of 4 adjacent output columns
   int gu = 1;
   for (int c = 0; c < res; c += 4) {
     if ((c % a.tc) + 4 > a.tc && (c % a.tc) % 4) continue;
@@ -898,8 +746,6 @@ int run_clip_preprocess(cb_ctx* ctx, const cb_surface_pool* pool, const int32_t*
   }
   a.gu = gu;
   if (ty->max_taps > 64 || tx->max_taps > 64) return fail(ctx, CB_ERR_UNSUPPORTED, "downscale factor too large (%d vertical taps)", ty->max_taps);
-  const char* kver = getenv("CB_PRE_KERNEL");
-  const bool use_v2 = !(kver && kver[0] == '1');
 
   rc = ensure_norm_lut(ctx, mean, std_, stream);
   if (rc) return rc;
@@ -909,8 +755,9 @@ int run_clip_preprocess(cb_ctx* ctx, const cb_surface_pool* pool, const int32_t*
 
   int max_slot = 0;
   for (int i = 0; i < n; ++i) max_slot = std::max(max_slot, (int)slots[i]);
-  // default: horizontal pass on the tensor pipe (preprocess_tc.cu); CB_PRE_KERNEL=2 / 1 select the SIMT generations for A/B
-  if (!kver || kver[0] == '3') {
+  // default: horizontal pass on the tensor pipe (preprocess_tc.cu), which returns 1 for plans it does not take
+  const char* kver = getenv("CB_PRE_KERNEL");
+  if (!kver || std::strcmp(kver, "2") != 0) {
     rc = run_clip_preprocess_tc(ctx, pool, a.slots, n, max_slot, res, out_mode, layout_patch, k_pad, dtype, tx, ty, out, stream);
     if (rc <= 0) return rc;
   }
@@ -939,7 +786,7 @@ int run_clip_preprocess(cb_ctx* ctx, const cb_surface_pool* pool, const int32_t*
   const int raw_stage = is_nv12(pool->format) ? (a.swa * kSR * 3 / 2) : (3 * a.swa * kSR);
   const int npx = out_mode == 2 ? a.tc / a.patch : 0;
   size_t smem = 2 * (size_t)raw_stage + (size_t)3 * kSR * (a.swa + 1) * 4 + (size_t)3 * a.ring * (a.tc | 1) * 4 + (size_t)npx * k_pad * 2 + 32;
-  if (use_v2) smem += 48 + (size_t)((a.tc + 3) / 4) * a.gu * 16 + (size_t)2 * ((a.tc + 3) / 4) * 4;
+  smem += 48 + (size_t)((a.tc + 3) / 4) * a.gu * 16 + (size_t)2 * ((a.tc + 3) / 4) * 4;
   if (smem > 227 * 1024) return fail(ctx, CB_ERR_UNSUPPORTED, "preprocess tile needs %zu bytes of shared memory", smem);
   dim3 grid(tiles, n);
   mark_launch(ctx, CB_PROF_PREPROCESS, stream);
@@ -948,15 +795,9 @@ int run_clip_preprocess(cb_ctx* ctx, const cb_surface_pool* pool, const int32_t*
     CB_CUDA(ctx, cudaFuncSetAttribute(KERNEL<F>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));               \
     KERNEL<F><<<grid, kThreads, smem, stream>>>(map_a, map_b, a);                                                        \
   } while (0)
-  if (use_v2) {
-    if (pool->format == CB_FMT_NV12) CB_LAUNCH_PRE(clip_preprocess_v2_kernel, CB_FMT_NV12);
-    else if (pool->format == CB_FMT_NV12_SWS) CB_LAUNCH_PRE(clip_preprocess_v2_kernel, CB_FMT_NV12_SWS);
-    else CB_LAUNCH_PRE(clip_preprocess_v2_kernel, CB_FMT_RGB24);
-  } else {
-    if (pool->format == CB_FMT_NV12) CB_LAUNCH_PRE(clip_preprocess_kernel, CB_FMT_NV12);
-    else if (pool->format == CB_FMT_NV12_SWS) CB_LAUNCH_PRE(clip_preprocess_kernel, CB_FMT_NV12_SWS);
-    else CB_LAUNCH_PRE(clip_preprocess_kernel, CB_FMT_RGB24);
-  }
+  if (pool->format == CB_FMT_NV12) CB_LAUNCH_PRE(clip_preprocess_v2_kernel, CB_FMT_NV12);
+  else if (pool->format == CB_FMT_NV12_SWS) CB_LAUNCH_PRE(clip_preprocess_v2_kernel, CB_FMT_NV12_SWS);
+  else CB_LAUNCH_PRE(clip_preprocess_v2_kernel, CB_FMT_RGB24);
 #undef CB_LAUNCH_PRE
   CB_CUDA(ctx, cudaGetLastError());
   return CB_OK;

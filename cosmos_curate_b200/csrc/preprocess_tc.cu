@@ -25,7 +25,6 @@
 // ~105 KB of shared memory per CTA: two CTAs per SM overlap each other's phases.  Output: u8 [n][3][res][res]; normalisation +
 // patch packing is a second, bandwidth-trivial kernel (pack_patches_kernel / normalize_pack_kernel) so that this one stays small.
 #include <algorithm>
-#include <cstdlib>
 #include <cstring>
 #include <vector>
 
@@ -42,10 +41,13 @@ constexpr int kRingStride = 3 * kNC + 4;  // floats per ring row: +16 B so that 
 constexpr int kMaxUnits = 128;            // units per frame column (4K: 55)
 constexpr int kVRows = 16, kVTaps = 40;   // vertical-pass weights of one unit staged in shared memory (rows x taps)
 constexpr int kTcThreads = 320;  // 10 warps: 20 row pairs x kw / 4 column groups of the convert phase divide evenly (kw = 128 / 192 / 256)
+// mbarrier waits suspend in hardware for up to this long instead of re-polling, which spares the co-resident CTA's issue
+// slots; spin, 32, 200 and 2000 ns measured the same
+constexpr int kWaitNs = 2000;
 
 struct TcArgs {
   const int* slots;
-  int n, res, ru, n_units, y_begin, kw, kb, colour, wait_ns;
+  int n, res, ru, n_units, y_begin, kw, kb, colour;
   int nc;                  // output columns per CTA slab: 32 (two N-tiles), or 16 when the downscale is so strong that 32 columns' window exceeds a TMA box
   const int* x_lo;         // [n_slabs] first source column of the slab window (multiple of 16)
   const int* tile_k0;      // [n_slabs * 2] first k-step (16 source columns) of the N-tile inside the window
@@ -195,8 +197,7 @@ __global__ void __launch_bounds__(kTcThreads, 2)
   };
   for (int u = 0; u < a.n_units; ++u) {
     if (u > 0) stage_taps(u - 1);  // for the vertical pass of the previous unit, which runs below while this unit's MMAs execute
-    if (a.wait_ns) mbar_wait_parked(raw_full, u & 1, a.wait_ns);
-    else mbar_wait(raw_full, u & 1);
+    mbar_wait_parked(raw_full, u & 1, kWaitNs);
     // ---- colour conversion straight into the A operand: a thread owns 2 rows x 4 pixels (two chroma samples)
     {
       const uint8_t* ry = sRaw;
@@ -278,8 +279,7 @@ __global__ void __launch_bounds__(kTcThreads, 2)
     }
     if (u > 0) vertical(u - 1);
     __syncthreads();  // the epilogue below overwrites ring rows the vertical pass was still reading
-    if (a.wait_ns) mbar_wait_parked(mma_done, u & 1, a.wait_ns);  // suspend-time hint: do not burn the co-resident CTA's issue slots
-    else mbar_wait(mma_done, u & 1);
+    mbar_wait_parked(mma_done, u & 1, kWaitNs);
     tc_fence_after();
     // ---- epilogue: the filtered rows of this unit -> ring (warp = lane quarter x N-tile)
     if (warp < 8) {
@@ -524,10 +524,6 @@ int run_clip_preprocess_tc(cb_ctx* ctx, const cb_surface_pool* pool, const int* 
   a.nc = p->nc;
   a.slots = d_slots, a.n = n, a.res = res, a.ru = p->ru, a.n_units = p->n_units, a.y_begin = p->y_begin, a.kw = p->kw, a.kb = p->kb;
   a.colour = pool->format;
-  {
-    const char* w = getenv("CB_PRE_WAIT_NS");  // A/B switch for the mbarrier waits: 0 = spin, else try_wait suspend-time hint in ns
-    a.wait_ns = w ? atoi(w) : 2000;
-  }
   a.x_lo = p->d_x_lo, a.tile_k0 = p->d_k0, a.tile_nk = p->d_nk, a.wtiles = p->d_w;
   a.ymin = ty->d_min, a.ysize = ty->d_size, a.unit_last = p->d_unit_last, a.wy = ty->d_w, a.ty = ty->max_taps, a.out = u8;
   const int b_tile = (p->kb / 64) * 4096;

@@ -7,8 +7,6 @@
 //   clip_tail_kernel       post_layernorm(CLS) -> visual_projection -> L2 normalise -> aesthetic affine head
 #include <cuda_fp16.h>
 
-#include <cstdlib>
-
 #include <type_traits>
 
 #include "common.h"
@@ -530,17 +528,10 @@ int layernorm_f16(cb_ctx* ctx, const float* x, const float* gamma, const float* 
   if (d % 128 || d > 128 * kLnMaxChunks) return fail(ctx, CB_ERR_UNSUPPORTED, "layernorm: d=%d must be a multiple of 128 and <= %d", d, 128 * kLnMaxChunks);
   mark_launch(ctx, CB_PROF_LAYERNORM, stream);
   const unsigned grid = (unsigned)((rows + 7) / 8);
-  // A/B switch (profiles/r02_layernorm_ab.jsonl): 0 = generic instantiation (5.29 TB/s at 1024), 1 = row-length instantiations
-  // (6.55 TB/s = the measured copy bandwidth; default), 2 = + 4 blocks per SM at 1024 (64 registers, 28 B spilled: 6.47 TB/s)
-  const char* ln_env = std::getenv("CB_LN_VARIANT");
-  const int variant = ln_env ? std::atoi(ln_env) : 1;
-  const int chunks = variant == 0 ? 0 : d >> 7;
-  switch (chunks) {  // ViT-B 768, ViT-L 1024, SoViT-400m 1152
+  // one instantiation per tower width reaches copy bandwidth, the generic one 81-88 % of it (profiles/r02_layernorm_ab.jsonl)
+  switch (d >> 7) {  // ViT-B 768, ViT-L 1024, SoViT-400m 1152
     case 6: layernorm_kernel<6, 4><<<grid, 256, 0, stream>>>(x, gamma, beta, (__half*)y, rows, d, eps); break;
-    case 8:
-      if (variant == 1) layernorm_kernel<8, 3><<<grid, 256, 0, stream>>>(x, gamma, beta, (__half*)y, rows, d, eps);
-      else layernorm_kernel<8, 4><<<grid, 256, 0, stream>>>(x, gamma, beta, (__half*)y, rows, d, eps);
-      break;
+    case 8: layernorm_kernel<8, 3><<<grid, 256, 0, stream>>>(x, gamma, beta, (__half*)y, rows, d, eps); break;
     case 9: layernorm_kernel<9, 3><<<grid, 256, 0, stream>>>(x, gamma, beta, (__half*)y, rows, d, eps); break;
     default: layernorm_kernel<0, 3><<<grid, 256, 0, stream>>>(x, gamma, beta, (__half*)y, rows, d, eps); break;
   }
@@ -558,17 +549,14 @@ int assemble_tokens(cb_ctx* ctx, const float* patch, const float* cls, const flo
   return CB_OK;
 }
 
-int attention_tc(cb_ctx* ctx, const void* qkv, void* out, int n, int tokens, int heads, int head_dim, cudaStream_t stream, bool* launched);
 int attention_tc2(cb_ctx* ctx, const void* qkv, void* out, int n, int tokens, int heads, int head_dim, cudaStream_t stream, bool* launched);
 
 int attention_f16(cb_ctx* ctx, const void* qkv, void* out, int n, int tokens, int heads, int head_dim, cudaStream_t stream) {
   if (!qkv || !out) return fail(ctx, CB_ERR_ARG, "attention: null operand");
   if (n <= 0) return CB_OK;
-  {  // head_dim 64, 129..257 tokens (ViT-L/14): tcgen05 kernel (attention_tc.cu); everything else: mma.sync kernel below
+  {  // head_dim 64, 129..257 tokens (ViT-L/14): tcgen05 kernel (attention_tc2.cu; CB_ATTN_KERNEL=mma skips it); everything else: mma.sync kernel below
     bool launched = false;
-    int rc = attention_tc2(ctx, qkv, out, n, tokens, heads, head_dim, stream, &launched);  // two threads per row (CB_ATTN_KERNEL=tc1|mma skips it)
-    if (rc || launched) return rc;
-    rc = attention_tc(ctx, qkv, out, n, tokens, heads, head_dim, stream, &launched);  // one thread per row
+    const int rc = attention_tc2(ctx, qkv, out, n, tokens, heads, head_dim, stream, &launched);
     if (rc || launched) return rc;
   }
   if (tokens <= 0 || heads <= 0 || head_dim % 8 || head_dim > 80 || head_dim < 16)

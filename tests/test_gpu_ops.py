@@ -82,21 +82,18 @@ def test_attention(ctx, n, t, heads, hd):
 
 
 def test_attention_tcgen05_and_mma_kernels_agree(ctx, monkeypatch):
-    """head_dim 64 / 129..257 tokens runs on tcgen05 (attention_tc.cu); CB_ATTN_KERNEL=mma forces the mma.sync kernel."""
+    """head_dim 64 / 129..257 tokens runs on tcgen05 (attention_tc2.cu); CB_ATTN_KERNEL=mma forces the mma.sync kernel."""
     g = torch.Generator(device="cuda").manual_seed(11)
     qkv = (torch.randn(20, 257, 3 * 1024, device="cuda", generator=g) * 2.0).half()
     qkv[:, :, 5] += 6.0  # a dominant query/key channel: sharp softmax rows
     tc = ctx.attention(qkv, 16).float()
-    monkeypatch.setenv("CB_ATTN_KERNEL", "tc1")  # first-generation tcgen05 kernel (one thread per row)
-    tc1 = ctx.attention(qkv, 16).float()
-    torch.testing.assert_close(tc, tc1, rtol=2e-3, atol=1e-3)
     monkeypatch.setenv("CB_ATTN_KERNEL", "mma")
     mma = ctx.attention(qkv, 16).float()
     torch.testing.assert_close(tc, mma, rtol=1e-2, atol=4e-3)
     again = ctx.attention(qkv, 16).float()
     assert torch.equal(mma, again)
     monkeypatch.delenv("CB_ATTN_KERNEL")
-    # The second-generation kernel issues a tile's four P.V chunk products in the fixed order 0, 2, 1, 3: repeat runs are bitwise equal
+    # The tcgen05 kernel issues a tile's four P.V chunk products in the fixed order 0, 2, 1, 3: repeat runs are bitwise equal
     # (also under load: 300 units per CTA-wave with different arrival timing of the two half-row streams).
     for _ in range(3):
         assert torch.equal(tc, ctx.attention(qkv, 16).float())
